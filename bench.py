@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200 worker decode engine (contract: DESIGN.md §6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): "decode tokens/sec/GPU (Llama-3-8B, seq 4K) + box req/s at 1/2/4/8 peers".
 
@@ -445,6 +445,11 @@ def run_ours(args):
     grp.barrier()
     clocks = clk.stop()
     launches = e.stats()["kernel_launches"] - launches0
+    if args.dump_outputs and rank == 0:
+        # what cl_decode_greedy returned for the timed steps; prompt, weights and warm-up depend only on the arguments
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        np.save(out_dir / "decode_ids.npy", out_ids.astype(np.float64))
     ms_max = grp.max(ms)
     value = n_gpus * K / (ms_max * 1e-3)
     mean_ctx = ctx + W + K / 2.0
@@ -574,11 +579,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-box", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the token ids of the timed decode steps to DIR/decode_ids.npy (float64), to compare two builds")
     ap.add_argument("--box-client", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--box-shard", default="", help=argparse.SUPPRESS)
     ap.add_argument("--workers", type=int, default=1, help=argparse.SUPPRESS)
     ap.add_argument("--base-port", type=int, default=21001, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU decode path computed; it needs --impl ours")
     if args.box_client:
         return run_box_client(args)
     return run_reference(args) if args.impl == "reference" else run_ours(args)

@@ -5,8 +5,12 @@ envelope with a mock engine (mirrors /root/reference/pkg/ipc/ipc_test.go:44-146)
 import collections
 import io
 import json
+import os
 import random
 import re
+import subprocess
+import sys
+import zlib
 from pathlib import Path
 
 import numpy as np
@@ -48,16 +52,26 @@ def test_presets_and_defaults():
     assert g.temperature == 0 and g.max_new_tokens == 5
 
 
+_NO_DEVICE_CHILD = """
+import numpy as np
+from crowdllama_b200 import engine as eng
+assert eng.device_count() == 0
+for call in (lambda: eng.Engine(preset="tiny-test"), lambda: eng.op_gemv(np.zeros((2, 16), np.uint16), np.zeros(16, np.float32))):
+    try:
+        call()
+    except eng.EngineError as ex:
+        assert ex.status == eng.CL_ERR_NO_DEVICE, ex.status
+    else:
+        raise AssertionError("the call succeeded without a device")
+"""
+
+
 def test_no_cpu_fallback():
-    """Without a device the product path must fail loudly (never route to the oracle)."""
-    if eng.device_count() > 0:
-        pytest.skip("GPU present")
-    with pytest.raises(eng.EngineError) as ei:
-        eng.Engine(preset="tiny-test")
-    assert ei.value.status == eng.CL_ERR_NO_DEVICE
-    with pytest.raises(eng.EngineError) as ei:
-        eng.op_gemv(np.zeros((2, 16), np.uint16), np.zeros(16, np.float32))
-    assert ei.value.status == eng.CL_ERR_NO_DEVICE
+    """Without a device the product path must fail loudly (never route to the oracle).  The device-facing calls run in
+    a child process that sees no GPU, so the check holds on machines with and without one."""
+    r = subprocess.run([sys.executable, "-c", _NO_DEVICE_CHILD], cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""},
+                       capture_output=True, text=True, timeout=120)
+    assert r.returncode == 0, r.stderr[-2000:]
     src = "".join(p.read_text() for p in (ROOT / "crowdllama_b200").rglob("*.py"))
     assert "oracle" not in src.replace("oracle oc_sample", "").replace("the oracle", "")
 
@@ -464,7 +478,7 @@ def test_sampler_stages_match_hf_logits_processors(case):
     repository's: support set and probabilities of the HF transformers processors applied in the same order.  8000
     draws per case over a 64-token vocabulary: no draw outside HF's support, every token's frequency within 5 sigma."""
     from oracle import oracle as oc
-    rng = np.random.default_rng(hash(tuple(sorted(case.items()))) % (2 ** 32))
+    rng = np.random.default_rng(zlib.crc32(repr(sorted(case.items())).encode()))   # hash() of a str varies per process
     V, n = 64, 8000
     lg = (rng.standard_normal(V) * 2.0).astype(np.float32)
     hist = [int(x) for x in rng.integers(0, V, size=case["hist"])]
