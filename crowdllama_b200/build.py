@@ -22,7 +22,7 @@ LIB = HERE / "lib" / "libclengine.so"
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 HOSTCXX = "/usr/bin/g++"
 
-SOURCES = ["decode_kernels.cu", "decode_mega.cu", "decode_mega_batch.cu", "attn_decode_tc.cu", "batch_kernels.cu", "engine.cu", "ops_api.cu", "prefill.cu", "gemm_tcgen05.cu", "prefill_kernels.cu", "attn_prefill_tc.cu",
+SOURCES = ["decode_kernels.cu", "decode_mega.cu", "decode_mega_batch.cu", "attn_decode_tc.cu", "batch_kernels.cu", "engine.cu", "ops_api.cu", "prefill.cu", "gemm_tcgen05.cu", "prefill_kernels.cu", "attn_prefill_tc.cu", "sample_kernels.cu",
            "host_util.cpp", "tokenizer.cpp", "weights_io.cpp", "scheduler.cpp", "capi.cpp"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-ccbin", HOSTCXX,
          "-Xcompiler", "-fPIC,-Wall,-Wno-unused-function,-fvisibility=default", "--expt-relaxed-constexpr",

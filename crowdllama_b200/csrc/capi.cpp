@@ -431,6 +431,12 @@ int cl_decode_greedy_batch(cl_engine* e, const cl_seq_t* seqs, int32_t n_seqs, c
   std::lock_guard<std::mutex> lk(e->impl.mu_);
   CL_GUARD(return e->impl.decode_greedy(seqs, n_seqs, first_ids, n_steps, ids_out, device_ms);)
 }
+int cl_decode_sample_batch(cl_engine* e, const cl_seq_t* seqs, int32_t n_seqs, const int32_t* first_ids, const cl_sampling* s,
+                           const uint64_t* first_steps, int32_t n_steps, int32_t* ids_out, float* device_ms) {
+  if (!e || !seqs || !first_ids || !s || !first_steps || !ids_out) return CL_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lk(e->impl.mu_);
+  CL_GUARD(return e->impl.decode_sample(seqs, n_seqs, first_ids, s, first_steps, n_steps, ids_out, device_ms);)
+}
 int cl_decode_step_batch(cl_engine* e, const cl_seq_t* seqs, int32_t n_seqs, const int32_t* ids, float* logits_out, int32_t* argmax_out) {
   if (!e || !seqs || !ids) return CL_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lk(e->impl.mu_);

@@ -185,6 +185,7 @@ int Engine::init(const cl_engine_config& c) {
   }
   // defaults of the round-2 features: see kDefault* in engine.h (flipped on once a GPU run has validated them)
   sched_prefill_chunk_ = env_int("CL_SCHED_PREFILL_CHUNK", kDefaultSchedPrefillChunk);
+  device_sample_ = env_int("CL_SCHED_DEVICE_SAMPLE", kDefaultSchedDeviceSample) != 0 && sample_nblk_ > 0;
   if (sched_prefill_chunk_ > 0 && sched_prefill_chunk_ < 16) sched_prefill_chunk_ = 16;
   prefill_small_max_ = std::min(256, env_int("CL_PREFILL_SMALL_MAX", kDefaultPrefillSmallMax));
   prefill_fused_ = env_int("CL_PREFILL_FUSED", kDefaultPrefillFused);
@@ -395,6 +396,15 @@ int Engine::alloc_state() {
   CL_CUDA_OK(cudaMemsetAsync(d_step_counter_, 0, 4, stream_));
   CL_CUDA_OK(cudaMallocHost(&h_logits_pinned_, (size_t)cfg.vocab_size * 4));
   CL_CUDA_OK(cudaMallocHost(&h_ids_pinned_, (size_t)ring_steps_ * max_batch_ * 4));
+  sample_nblk_ = sample_blocks(cfg.vocab_size);
+  if (sample_nblk_ > 0) {
+    DMALLOC(d_sample_state_, S * sizeof(SampleSlot));
+    DMALLOC(d_sample_part_, S * sample_nblk_ * kSampleCand * sizeof(unsigned long long));
+    DMALLOC(d_sample_cnt_, S * 4);
+    DMALLOC(d_sample_slots_, S * 4);
+    CL_CUDA_OK(cudaMemsetAsync(d_sample_state_, 0, S * sizeof(SampleSlot), stream_));
+    CL_CUDA_OK(cudaMemsetAsync(d_sample_cnt_, 0, S * 4, stream_));
+  }
   return CL_OK;
 }
 
@@ -402,6 +412,7 @@ int Engine::alloc_state() {
 int Engine::seq_create(cl_seq_t* out) {
   for (int i = 0; i < max_seqs_; ++i)
     if (!seqs_[i].live) {
+      if (d_sample_state_) CL_CUDA_OK(cudaMemsetAsync(d_sample_state_ + i, 0, sizeof(SampleSlot), stream_));   // off the device sampler
       seqs_[i] = SeqState();
       seqs_[i].live = true;
       *out = i;
@@ -810,6 +821,12 @@ int Engine::prefill(cl_seq_t s, const int32_t* ids, int n, float* logits_out) {
 }
 
 int Engine::decode_greedy(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms) {
+  return decode_loop(ss, B, first_ids, n_steps, ids_out, device_ms, false);
+}
+
+// n_steps batched steps on the device; with `sample`, the sampler runs after every step (slots set up by sample_setup)
+int Engine::decode_loop(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms,
+                        bool sample) {
   if (B <= 0 || B > max_batch_ || n_steps <= 0) { set_last_error("bad batch / steps"); return CL_ERR_INVALID_ARG; }
   for (int b = 0; b < B; ++b) {
     const int s = ss[b];
@@ -833,7 +850,8 @@ int Engine::decode_greedy(const cl_seq_t* ss, int B, const int32_t* first_ids, i
     CL_CUDA_OK(cudaMemsetAsync(d_step_counter_, 0, 4, stream_));
     CL_CUDA_OK(cudaEventRecord(ev0_, stream_));
     for (int i = 0; i < chunk; ++i) {
-      const int rc = run_step_graph(B);
+      int rc = run_step_graph(B);
+      if (rc == CL_OK && sample) rc = launch_sampler(B, d_slots_, true);
       if (rc) return rc;
     }
     CL_CUDA_OK(cudaEventRecord(ev1_, stream_));
@@ -859,6 +877,83 @@ int Engine::decode_greedy(const cl_seq_t* ss, int B, const int32_t* first_ids, i
   }
   if (device_ms) *device_ms = total_ms;
   return CL_OK;
+}
+
+// ---- device sampler (sample_kernels.cu) -------------------------------------------------------------
+bool Engine::sample_qualifies(const cl_sampling& sp, int vocab) {
+  const bool penalty = sp.repeat_penalty != 1.0f && sp.repeat_last_n != 0;
+  return sp.temperature > 0.f && sp.top_k >= 1 && sp.top_k <= CL_SAMPLE_MAX_TOP_K && sp.top_k < vocab &&
+         (!penalty || (sp.repeat_last_n > 0 && sp.repeat_last_n <= CL_SAMPLE_MAX_WINDOW));
+}
+
+SampleSlot Engine::sample_slot(const cl_sampling& sp, int vocab, const int32_t* hist, int n_hist, uint64_t step) {
+  SampleSlot h;
+  if (!sample_qualifies(sp, vocab)) return h;
+  h.temperature = sp.temperature; h.top_p = sp.top_p; h.penalty = sp.repeat_penalty; h.top_k = sp.top_k;
+  h.seed = sp.seed; h.step = step;
+  if (sp.repeat_penalty != 1.0f && sp.repeat_last_n != 0) {
+    h.win_len = sp.repeat_last_n;   // an empty history leaves the window to fill with the drawn ids
+    h.win_count = hist ? std::min(std::max(n_hist, 0), h.win_len) : 0;
+    for (int j = 0; j < h.win_count; ++j) h.win[j] = hist[n_hist - h.win_count + j];
+  }
+  return h;
+}
+
+int Engine::sample_setup(cl_seq_t s, const cl_sampling& sp, const int32_t* hist, int n_hist, uint64_t step) {
+  if (!d_sample_state_) { set_last_error("vocabulary too large for the device sampler"); return CL_ERR_INVALID_ARG; }
+  const SampleSlot h = sample_slot(sp, cfg.vocab_size, hist, n_hist, step);
+  CL_CUDA_OK(cudaMemcpyAsync(d_sample_state_ + s, &h, sizeof h, cudaMemcpyHostToDevice, stream_));
+  return CL_OK;
+}
+
+int Engine::launch_sampler(int B, const int* d_slots, bool ring) {
+  SampleArgs a;
+  a.logits = d_logits_; a.vocab = cfg.vocab_size; a.state = d_sample_state_; a.tok = d_tok_;
+  if (ring) { a.ids_ring = d_ids_ring_; a.step_counter = d_step_counter_; a.ring_steps = ring_steps_; a.ring_stride = max_batch_; }
+  a.part = d_sample_part_; a.counters = d_sample_cnt_; a.slots = d_slots; a.batch = B; a.nblk = sample_nblk_;
+  const int n = launch_sample(a, stream_);
+  if (n < 0) { set_last_error(std::string("launch_sample: ") + cudaGetErrorString(cudaGetLastError())); return CL_ERR_CUDA; }
+  launches_ += n;
+  return CL_OK;
+}
+
+int Engine::sample_slots(const cl_seq_t* ss, int n, int32_t* ids_out) {
+  if (n <= 0) return CL_OK;
+  if (!d_sample_state_ || n > max_seqs_) { set_last_error("sample_slots: bad slot list"); return CL_ERR_INVALID_ARG; }
+  CL_CUDA_OK(cudaMemcpyAsync(d_sample_slots_, ss, (size_t)n * 4, cudaMemcpyHostToDevice, stream_));
+  int rc = launch_sampler(n, d_sample_slots_, false);
+  if (rc || !ids_out) return rc;
+  CL_CUDA_OK(cudaMemcpyAsync(h_ids_pinned_, d_tok_, (size_t)max_seqs_ * 4, cudaMemcpyDeviceToHost, stream_));
+  CL_CUDA_OK(cudaStreamSynchronize(stream_));
+  for (int i = 0; i < n; ++i) ids_out[i] = h_ids_pinned_[ss[i]];
+  return CL_OK;
+}
+
+int Engine::decode_sample(const cl_seq_t* ss, int B, const int32_t* first_ids, const cl_sampling* sps, const uint64_t* first_steps,
+                          int n_steps, int32_t* ids_out, float* device_ms) {
+  if (B <= 0 || B > max_batch_ || n_steps <= 0) { set_last_error("bad batch / steps"); return CL_ERR_INVALID_ARG; }
+  if (!d_sample_state_) { set_last_error("vocabulary too large for the device sampler"); return CL_ERR_INVALID_ARG; }
+  bool any = false;
+  for (int b = 0; b < B; ++b) {
+    const int s = ss[b];
+    if (s < 0 || s >= max_seqs_ || !seqs_[s].live) return CL_ERR_BAD_SEQ;
+    if (sps[b].temperature > 0.f && !sample_qualifies(sps[b], cfg.vocab_size)) {
+      set_last_error("sampling options outside the device sampler's limits (CL_SAMPLE_MAX_TOP_K / CL_SAMPLE_MAX_WINDOW)");
+      return CL_ERR_INVALID_ARG;
+    }
+    any = any || sps[b].temperature > 0.f;
+  }
+  std::vector<int32_t> hist;
+  for (int b = 0; b < B; ++b) {
+    if (first_ids[b] < 0 || first_ids[b] >= cfg.vocab_size) break;   // decode_loop reports it
+    const auto& h = seqs_[ss[b]].history;
+    const size_t keep = std::min<size_t>(h.size(), CL_SAMPLE_MAX_WINDOW);
+    hist.assign(h.end() - keep, h.end());
+    hist.push_back(first_ids[b]);
+    const int rc = sample_setup(ss[b], sps[b], hist.data(), (int)hist.size(), first_steps[b]);
+    if (rc) return rc;
+  }
+  return decode_loop(ss, B, first_ids, n_steps, ids_out, device_ms, any);
 }
 
 // ---- parity / benchmark aids ------------------------------------------------------------------------

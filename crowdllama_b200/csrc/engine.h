@@ -26,6 +26,7 @@ constexpr int kDefaultPrefillFused = 1;         // CL_PREFILL_FUSED bit mask: 1 
 constexpr int kDefaultSchedMultiPrefill = 1;    // CL_SCHED_MULTI_PREFILL: scheduler admits the prompts at the head of the queue in one tile-path pass (Engine::prefill_multi; validated r2v: 64 clients x 146-token prompts 38.5 -> 47.4 req/s)
 constexpr int kDefaultSchedLingerUs = 1000;     // CL_SCHED_LINGER_US: with an empty batch, keep collecting while requests arrive within this gap (max 8x in total)
 constexpr int kDefaultBatchMega = 0;            // CL_BATCH_MEGA: persistent batched decode kernel for B >= 2
+constexpr int kDefaultSchedDeviceSample = 1;    // CL_SCHED_DEVICE_SAMPLE: requests within the device sampler's limits are sampled on the GPU (sample_kernels.cu); validated r3a: Ollama-default traffic at max_batch 64 21.3 -> 84.7 req/s
 
 void set_last_error(const std::string& s);
 const char* get_last_error();
@@ -157,6 +158,19 @@ class Engine {
   int decode_step(cl_seq_t s, int32_t id, float* logits_out, int32_t* argmax_out);
   int decode_greedy(const cl_seq_t* seqs, int n_seqs, const int32_t* first_ids, int n_steps, int32_t* ids_out,
                     float* device_ms);
+  // sampled counterpart: step graph + device sampler per step; sps[b] greedy or within the device limits
+  int decode_sample(const cl_seq_t* seqs, int n_seqs, const int32_t* first_ids, const cl_sampling* sps, const uint64_t* first_steps,
+                    int n_steps, int32_t* ids_out, float* device_ms);
+  // device sampler (sample_kernels.cu): true if the request's options fit its limits (clengine.h CL_SAMPLE_MAX_*)
+  static bool sample_qualifies(const cl_sampling& sp, int vocab);
+  // the sampler state of one slot (top_k 0: not sampled on the device); window = the last repeat_last_n ids of hist
+  static SampleSlot sample_slot(const cl_sampling& sp, int vocab, const int32_t* hist, int n_hist, uint64_t step);
+  // upload slot s's sampler state: the draw counter `step` and the penalty window = the last repeat_last_n ids of
+  // hist[0, n_hist) (the history the next draw sees).  A greedy or non-qualifying sp leaves the slot off the sampler.
+  int sample_setup(cl_seq_t s, const cl_sampling& sp, const int32_t* hist, int n_hist, uint64_t step);
+  // draw the next token of the n slots whose last-position logits an admission has just left in d_logits_
+  // (d_tok_[slot] is overwritten); ids_out (host, may be nullptr) receives them
+  int sample_slots(const cl_seq_t* ss, int n, int32_t* ids_out);
   int set_tensor(int layer, int kind, const uint16_t* data, int64_t n);
   int load_safetensors(const std::string& path);   // HF llama-layout checkpoint (file or directory) -> set_tensor (weights_io.cpp)
   // parity / benchmark aids (token level)
@@ -180,6 +194,7 @@ class Engine {
   std::string model_name;
   std::mutex mu_;               // serialises every GPU-touching call
   std::unique_ptr<Tokenizer> tok;
+  bool device_sample_ = false;  // requests within the device sampler's limits are sampled on the GPU (CL_SCHED_DEVICE_SAMPLE)
 
  private:
   int alloc_weights();
@@ -192,6 +207,8 @@ class Engine {
   bool ensure_graph(int B);
   void precapture_graphs();                       // graph launch (or eager enqueue)
   int read_logits(int slot, float* out);
+  int launch_sampler(int B, const int* d_slots, bool ring);   // sampler over d_slots[0..B) (ring: write the step's ids_ring row)
+  int decode_loop(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms, bool sample);
   int prefill_tokenwise(cl_seq_t s, const int32_t* ids, int n, float* logits_out);
   int prefill_chunked(cl_seq_t s, const int32_t* ids, int n, float* logits_out);
   int ensure_prefill_ws(int tokens);  // tcgen05 path (prefill.cu)
@@ -238,6 +255,12 @@ class Engine {
   int* d_ids_ring_ = nullptr; int* d_step_counter_ = nullptr; int* d_prompt_ = nullptr;
   int ring_steps_ = 1024, prompt_cap_ = 0;
   float* h_logits_pinned_ = nullptr; int* h_ids_pinned_ = nullptr;
+  // device sampler (sample_kernels.cu)
+  SampleSlot* d_sample_state_ = nullptr;                 // [max_seqs]
+  unsigned long long* d_sample_part_ = nullptr;          // [max_seqs][sample_nblk_][kSampleCand]
+  unsigned* d_sample_cnt_ = nullptr;                     // [max_seqs]
+  int* d_sample_slots_ = nullptr;                        // [max_seqs] slot list of an admission's sampler launch
+  int sample_nblk_ = 0;                                  // 0: vocabulary too large for the device sampler
 
   // prefill workspace (allocated lazily)
   struct PrefillWs {

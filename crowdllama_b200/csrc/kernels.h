@@ -5,6 +5,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/clengine.h"
+
 namespace cl {
 
 // Dependencies inside the token step (common.cuh: wait_counter_warp / signal_counter).
@@ -98,6 +100,34 @@ struct StepTailArgs {                // argmax over logits, advance the sequence
   const int* slots = nullptr;
   int batch = 1;
 };
+
+// per-slot state of the device sampler (sample_kernels.cu).  The kernel advances `step` and the window after each draw.
+struct SampleSlot {
+  float temperature = 0.f, top_p = 0.f, penalty = 1.f;
+  int top_k = 0;                     // 0: the slot is not sampled on the device (greedy, or outside the device limits)
+  int win_len = 0;                   // repeat_last_n while the penalty is on, else 0
+  int win_count = 0;                 // ids appended so far: win[0, min(win_count, win_len)) hold the window, id j at j % win_len
+  unsigned long long seed = 0, step = 0;
+  int win[CL_SAMPLE_MAX_WINDOW] = {};
+};
+
+struct SampleArgs {
+  const float* logits = nullptr;     // [slot][vocab], read in place
+  int vocab = 0;
+  SampleSlot* state = nullptr;       // [slot]
+  int* tok = nullptr;                // [slot] next input token: overwritten for the sampled slots
+  int* ids_ring = nullptr;           // [ring_steps][ring_stride] (nullptr: not written) — entry of the step just run
+  const int* step_counter = nullptr; // already bumped by the step: the step's ring row is (*step_counter - 1) % ring_steps
+  int ring_steps = 0, ring_stride = 0;
+  unsigned long long* part = nullptr;// [slot][nblk][kSampleCand] per-CTA candidate keys
+  unsigned* counters = nullptr;      // [slot] arrival counters (self re-arming)
+  const int* slots = nullptr;        // [batch] (nullptr: identity)
+  int batch = 1;
+  int nblk = 1;                      // CTAs per row: sample_blocks(vocab)
+};
+constexpr int kSampleCand = CL_SAMPLE_MAX_TOP_K + CL_SAMPLE_MAX_WINDOW;   // candidates one CTA keeps for the merge
+int sample_blocks(int vocab);        // CTAs per row; 0 if the vocabulary is too large for the sampler
+int launch_sample(const SampleArgs& a, cudaStream_t st);
 
 // every launcher returns the number of kernels it enqueued (for cl_stats.kernel_launches)
 int launch_gemv(int variant, int epi, bool norm, const GemvArgs& a, cudaStream_t st, bool pdl, int* n_ctas = nullptr);

@@ -216,6 +216,65 @@ int cl_op_qkv_rope_append(int device, int variant, const uint16_t* w_qkv, const 
   return CL_OK;
 }
 
+int cl_op_sample(int device, const float* logits, int32_t n_rows, int32_t vocab, const cl_sampling* s, const int32_t* windows,
+                 const int32_t* n_window, const uint64_t* steps, int32_t* ids_out, int32_t iters, float* ms) {
+  if (!logits || !s || !windows || !n_window || !steps || !ids_out || n_rows <= 0 || vocab <= 0) return CL_ERR_INVALID_ARG;
+  int rc = check_device(device);
+  if (rc) return rc;
+  const int nblk = sample_blocks(vocab);
+  if (!nblk) { set_last_error("vocabulary too large for the device sampler"); return CL_ERR_INVALID_ARG; }
+  std::vector<SampleSlot> state((size_t)n_rows);
+  for (int r = 0; r < n_rows; ++r) {
+    const cl_sampling& sp = s[r];
+    const int nw = n_window[r];
+    if (!Engine::sample_qualifies(sp, vocab) || nw < 0 || nw > CL_SAMPLE_MAX_WINDOW) {
+      set_last_error("row " + std::to_string(r) + ": outside the device sampler's limits");
+      return CL_ERR_INVALID_ARG;
+    }
+    state[r] = Engine::sample_slot(sp, vocab, windows + (size_t)r * CL_SAMPLE_MAX_WINDOW, nw, steps[r]);
+  }
+  const size_t row_bytes = (size_t)vocab * 4, bytes = (size_t)n_rows * row_bytes;
+  DevBuf dl, dst, dpart, dcnt, dtok;
+  CL_CUDA_OK(dl.upload(logits, bytes));
+  CL_CUDA_OK(dst.upload(state.data(), state.size() * sizeof(SampleSlot)));
+  CL_CUDA_OK(dpart.alloc((size_t)n_rows * nblk * kSampleCand * sizeof(unsigned long long)));
+  CL_CUDA_OK(dcnt.alloc((size_t)n_rows * 4));
+  CL_CUDA_OK(cudaMemset(dcnt.p, 0, (size_t)n_rows * 4));
+  CL_CUDA_OK(dtok.alloc((size_t)n_rows * 4));
+  SampleArgs a;
+  a.logits = dl.as<float>(); a.vocab = vocab; a.state = dst.as<SampleSlot>(); a.tok = dtok.as<int>();
+  a.part = dpart.as<unsigned long long>(); a.counters = dcnt.as<unsigned>(); a.batch = n_rows; a.nblk = nblk;
+  if (launch_sample(a, nullptr) < 0) { set_last_error(std::string("launch_sample: ") + cudaGetErrorString(cudaGetLastError())); return CL_ERR_CUDA; }
+  CL_CUDA_OK(cudaDeviceSynchronize());
+  CL_CUDA_OK(cudaMemcpy(ids_out, dtok.p, (size_t)n_rows * 4, cudaMemcpyDeviceToHost));
+  if (iters > 0 && ms) {
+    // timing loop over enough copies of the logits to exceed the 126 MB L2 (each launch reads rows no earlier launch left there)
+    const int copies = (int)std::min<size_t>(16, (256ull << 20) / bytes + 1);
+    std::vector<DevBuf> extra(copies > 1 ? copies - 1 : 0);
+    std::vector<const float*> ls{dl.as<float>()};
+    for (auto& b : extra) {
+      CL_CUDA_OK(b.alloc(bytes));
+      CL_CUDA_OK(cudaMemcpy(b.p, dl.p, bytes, cudaMemcpyDeviceToDevice));
+      ls.push_back(b.as<float>());
+    }
+    cudaEvent_t e0, e1;
+    CL_CUDA_OK(cudaEventCreate(&e0));
+    CL_CUDA_OK(cudaEventCreate(&e1));
+    for (int i = 0; i < 3; ++i) { a.logits = ls[i % ls.size()]; launch_sample(a, nullptr); }
+    CL_CUDA_OK(cudaDeviceSynchronize());
+    CL_CUDA_OK(cudaEventRecord(e0, nullptr));
+    for (int i = 0; i < iters; ++i) { a.logits = ls[i % ls.size()]; launch_sample(a, nullptr); }
+    CL_CUDA_OK(cudaEventRecord(e1, nullptr));
+    CL_CUDA_OK(cudaDeviceSynchronize());
+    float t = 0.f;
+    CL_CUDA_OK(cudaEventElapsedTime(&t, e0, e1));
+    *ms = t / (float)iters;
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+  }
+  return CL_OK;
+}
+
 int cl_op_synth_weights(int device, uint64_t seed, int32_t tensor_key, int64_t n, float scale, uint16_t* out_bf16) {
   if (!out_bf16 || n <= 0) return CL_ERR_INVALID_ARG;
   int rc = check_device(device);

@@ -39,6 +39,7 @@ struct Request {
   uint64_t arrival = 0;
   std::vector<int32_t> full;        // prompt + tokens generated before a preemption: what the (re-)prefill has to process
   size_t prefilled = 0;             // tokens of `full` already in the cache (chunked admission)
+  bool dev_sample = false;          // sampled on the device (Engine::sample_qualifies and CL_SCHED_DEVICE_SAMPLE), set at admission
   bool greedy() const { return sp.temperature <= 0.f; }
 };
 
@@ -86,22 +87,33 @@ static int generate_sync(Engine& e, Request& r, const Engine::TokenSink* sink) {
   const int V = e.cfg.vocab_size;
   int rc = e.seq_create(&r.seq);
   if (rc) return rc;
+  // a sampled request within the device sampler's limits never copies logits to the host
+  r.dev_sample = e.device_sample_ && !r.greedy() && Engine::sample_qualifies(r.sp, V);
   std::vector<float> logits(V);
   int64_t t0 = now_ns();
-  rc = e.prefill(r.seq, r.prompt.data(), (int)r.prompt.size(), logits.data());
+  rc = e.prefill(r.seq, r.prompt.data(), (int)r.prompt.size(), r.dev_sample ? nullptr : logits.data());
   r.prefill_ns = now_ns() - t0;
   if (rc) { e.seq_free(r.seq); return rc; }
   t0 = now_ns();
   std::vector<int32_t> hist(r.prompt);
-  int32_t next = sample_token(logits.data(), V, r.sp, hist.data(), (int)hist.size(), 0);
+  int32_t next = 0;
+  if (r.dev_sample) {
+    rc = e.sample_setup(r.seq, r.sp, r.prompt.data(), (int)r.prompt.size(), 0);
+    if (rc == CL_OK) rc = e.sample_slots(&r.seq, 1, &next);
+    if (rc) { e.seq_free(r.seq); return rc; }
+  } else {
+    next = sample_token(logits.data(), V, r.sp, hist.data(), (int)hist.size(), 0);
+  }
   r.out.push_back(next);
   emit();
   while (!finished(r, *e.tok, e.cfg.max_seq_len)) {
-    if (r.greedy()) {
+    if (r.greedy() || r.dev_sample) {
       int room = std::min(r.max_new - (int)r.out.size(), e.cfg.max_seq_len - (int)(r.prompt.size() + r.out.size()));
       int chunk = std::min(room, sink ? 8 : 32);
       std::vector<int32_t> ids(chunk);
-      rc = e.decode_greedy(&r.seq, 1, &next, chunk, ids.data(), nullptr);
+      const uint64_t step = (uint64_t)r.out.size();
+      rc = r.greedy() ? e.decode_greedy(&r.seq, 1, &next, chunk, ids.data(), nullptr)
+                      : e.decode_sample(&r.seq, 1, &next, &r.sp, &step, chunk, ids.data(), nullptr);
       if (rc) break;
       for (int i = 0; i < chunk; ++i) {
         r.out.push_back(ids[i]);
@@ -287,6 +299,18 @@ void Engine::scheduler_main() {
         if (rc == CL_OK) rc = prefill_multi((int)ss.size(), ss.data(), ptrs.data(), lens.data(), nullptr);
         const int64_t pdt = now_ns() - t0;
         if (rc == CL_OK) {
+          // first tokens of the device-sampled requests: one sampler launch over the group's logits rows
+          std::vector<cl_seq_t> dev;
+          for (auto& r : group) {
+            r->dev_sample = device_sample_ && !r->greedy() && sample_qualifies(r->sp, V);
+            if (!r->dev_sample) continue;
+            rc = sample_setup(r->seq, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
+            if (rc) break;
+            dev.push_back(r->seq);
+          }
+          if (rc == CL_OK) rc = sample_slots(dev.data(), (int)dev.size(), nullptr);
+        }
+        if (rc == CL_OK) {
           cudaMemcpyAsync(toks.data(), d_tok_, (size_t)max_seqs_ * 4, cudaMemcpyDeviceToHost, stream_);
           if (cudaStreamSynchronize(stream_) != cudaSuccess) rc = CL_ERR_CUDA;
         }
@@ -298,8 +322,8 @@ void Engine::scheduler_main() {
           for (auto& r : group) {
             r->prefill_ns += pdt;
             r->prefilled = r->full.size();
-            int32_t next = toks[r->seq];                       // greedy: the device argmax of the pass
-            if (!r->greedy()) {
+            int32_t next = toks[r->seq];                       // greedy: the device argmax of the pass; device-sampled: the draw
+            if (!r->greedy() && !r->dev_sample) {
               read_logits(r->seq, logits.data());
               next = sample_token(logits.data(), V, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
               cudaMemcpyAsync(d_tok_ + r->seq, &next, 4, cudaMemcpyHostToDevice, stream_);
@@ -345,6 +369,7 @@ void Engine::scheduler_main() {
             if (rc == CL_OK) rc = ensure_capacity(r->seq, (int)r->full.size() + 1);   // all pages up front: a later chunk cannot run dry
             if (rc) { if (r->seq >= 0) seq_free(r->seq); r->seq = -1; complete(r, rc, get_last_error()); continue; }
             r->prefilled = 0;
+            r->dev_sample = device_sample_ && !r->greedy() && sample_qualifies(r->sp, V);
             prefilling_ = r;
           }
         }
@@ -361,7 +386,7 @@ void Engine::scheduler_main() {
       const size_t chunk = active_.empty() ? left : std::min(left, (size_t)budget);   // nobody to stall: the whole prompt at once
       const bool last = chunk == left;
       const int64_t t0 = now_ns();
-      const int rc = prefill(r->seq, r->full.data() + r->prefilled, (int)chunk, last ? logits.data() : nullptr);
+      int rc = prefill(r->seq, r->full.data() + r->prefilled, (int)chunk, last && !r->dev_sample ? logits.data() : nullptr);
       const int64_t pdt = now_ns() - t0;
       r->prefill_ns += pdt;
       sched_prefill_calls_++; sched_prefill_tokens_ += (int64_t)chunk; sched_prefill_ns_ += pdt;
@@ -371,10 +396,17 @@ void Engine::scheduler_main() {
       r->prefilled += chunk;
       if (!last) break;                   // budget used up in the middle of a prompt
       prefilling_.reset();
-      const int32_t next = sample_token(logits.data(), V, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
+      int32_t next = 0;
+      if (r->dev_sample) {
+        rc = sample_setup(r->seq, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
+        if (rc == CL_OK) rc = sample_slots(&r->seq, 1, &next);
+        if (rc) { seq_free(r->seq); r->seq = -1; complete(r, rc, get_last_error()); continue; }
+      } else {
+        next = sample_token(logits.data(), V, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
+      }
       r->out.push_back(next);
       publish(*r, next);
-      if (!r->greedy()) cudaMemcpyAsync(d_tok_ + r->seq, &r->out.back(), 4, cudaMemcpyHostToDevice, stream_);
+      if (!r->greedy() && !r->dev_sample) cudaMemcpyAsync(d_tok_ + r->seq, &r->out.back(), 4, cudaMemcpyHostToDevice, stream_);
       if (finished(*r, *tok, cfg.max_seq_len)) {
         seq_free(r->seq);
         requests_completed_++;
@@ -437,6 +469,9 @@ void Engine::scheduler_main() {
     }
     const int64_t t0 = now_ns();
     int rc = run_step_graph(B);
+    // the device sampler overwrites the step's argmax of the device-sampled slots (one launch for the whole batch)
+    if (rc == CL_OK && std::any_of(active_.begin(), active_.end(), [](const std::shared_ptr<Request>& r) { return r->dev_sample; }))
+      rc = launch_sampler(B, d_slots_, false);
     if (rc == CL_OK) {
       cudaMemcpyAsync(toks.data(), d_tok_, (size_t)max_seqs_ * 4, cudaMemcpyDeviceToHost, stream_);
       // Batched steps last 3.5-6 ms: wait on a blocking-sync event instead of spinning in cudaStreamSynchronize, so that
@@ -459,7 +494,7 @@ void Engine::scheduler_main() {
       st.history.push_back(r->out.back());
       st.len += 1;
       int32_t next = toks[r->seq];
-      if (!r->greedy()) {
+      if (!r->greedy() && !r->dev_sample) {
         read_logits(r->seq, logits.data());
         next = sample_token(logits.data(), V, r->sp, st.history.data(), (int)st.history.size(), (uint64_t)r->out.size());
         cudaMemcpyAsync(d_tok_ + r->seq, &next, 4, cudaMemcpyHostToDevice, stream_);

@@ -18,6 +18,10 @@ CL_OK = 0
 CL_ERR_INVALID_ARG, CL_ERR_NO_DEVICE, CL_ERR_CUDA, CL_ERR_OOM, CL_ERR_UNKNOWN_MODEL, CL_ERR_TOO_LONG, \
     CL_ERR_BAD_SEQ, CL_ERR_SHUTDOWN, CL_ERR_IO, CL_ERR_INTERNAL, CL_ERR_BAD_MESSAGE = range(-1, -12, -1)
 
+# device sampler limits (include/clengine.h CL_SAMPLE_MAX_TOP_K / CL_SAMPLE_MAX_WINDOW)
+SAMPLE_MAX_TOP_K = 128
+SAMPLE_MAX_WINDOW = 64
+
 KINDS = dict(EMBED=0, LM_HEAD=1, FINAL_NORM=2, ATTN_NORM=3, WQ=4, WK=5, WV=6, WO=7, FFN_NORM=8, WGATE=9, WUP=10,
              WDOWN=11)
 
@@ -68,10 +72,10 @@ EXPORTS = [
     "cl_greedy_sampling", "cl_sample_token", "cl_model_preset", "cl_engine_create", "cl_engine_destroy", "cl_engine_model_config",
     "cl_engine_stats", "cl_engine_set_tensor", "cl_checkpoint_info", "cl_generate", "cl_generate_ids", "cl_generate_stream", "cl_result_free",
     "cl_handle_message", "cl_handle_message_stream", "cl_buffer_free", "cl_tokenize", "cl_detokenize", "cl_seq_create", "cl_seq_free",
-    "cl_seq_len", "cl_prefill", "cl_prefill_batch", "cl_decode_step", "cl_decode_greedy", "cl_decode_greedy_batch", "cl_decode_step_batch", "cl_seq_fake_fill",
+    "cl_seq_len", "cl_prefill", "cl_prefill_batch", "cl_decode_step", "cl_decode_greedy", "cl_decode_greedy_batch", "cl_decode_sample_batch", "cl_decode_step_batch", "cl_seq_fake_fill",
     "cl_time_dominant_kernel", "cl_debug_kv", "cl_debug_hidden", "cl_debug_timeline",
     "cl_op_gemv", "cl_op_gemv_residual", "cl_op_rmsnorm_gemv", "cl_op_rmsnorm_gateup", "cl_op_qkv_rope_append", "cl_op_attn_decode",
-    "cl_op_gemm_bf16", "cl_op_attn_prefill", "cl_op_attn_prefill_variant", "cl_op_synth_weights", "cl_kvpool_create", "cl_kvpool_destroy",
+    "cl_op_gemm_bf16", "cl_op_attn_prefill", "cl_op_attn_prefill_variant", "cl_op_sample", "cl_op_synth_weights", "cl_kvpool_create", "cl_kvpool_destroy",
     "cl_kvpool_reserve", "cl_kvpool_release", "cl_kvpool_pages_of", "cl_kvpool_free_pages", "cl_kvpool_used_pages",
     "cl_tokenizer_load", "cl_tokenizer_free", "cl_tokenizer_encode", "cl_tokenizer_decode", "cl_tokenizer_info", "cl_engine_load_tokenizer",
 ]
@@ -126,6 +130,7 @@ def lib():
         "cl_decode_step": (C.c_int, [vp, i32, i32, vp, P(i32)]),
         "cl_decode_greedy": (C.c_int, [vp, i32, i32, i32, vp, P(f32)]),
         "cl_decode_greedy_batch": (C.c_int, [vp, vp, i32, vp, i32, vp, P(f32)]),
+        "cl_decode_sample_batch": (C.c_int, [vp, vp, i32, vp, P(Sampling), vp, i32, vp, P(f32)]),
         "cl_decode_step_batch": (C.c_int, [vp, vp, i32, vp, vp, vp]),
         "cl_seq_fake_fill": (C.c_int, [vp, i32, i32]),
         "cl_time_dominant_kernel": (C.c_int, [vp, i32, i32, i32, P(f32), P(f32)]),
@@ -141,6 +146,7 @@ def lib():
         "cl_op_gemm_bf16": (C.c_int, [C.c_int, vp, vp, vp, i32, i32, i32, i32, P(f32)]),
         "cl_op_attn_prefill": (C.c_int, [C.c_int, vp, vp, vp, i32, i32, i32, i32, vp]),
         "cl_op_attn_prefill_variant": (C.c_int, [C.c_int, C.c_int, vp, vp, vp, i32, i32, i32, i32, vp, i32, P(f32)]),
+        "cl_op_sample": (C.c_int, [C.c_int, vp, i32, i32, P(Sampling), vp, vp, vp, vp, i32, P(f32)]),
         "cl_op_synth_weights": (C.c_int, [C.c_int, u64, i32, i64, f32, vp]),
         "cl_tokenizer_load": (C.c_int, [C.c_char_p, C.c_char_p, P(vp)]),
         "cl_tokenizer_free": (None, [vp]),
@@ -350,6 +356,19 @@ class Engine:
         ms = C.c_float(0)
         _check(lib().cl_decode_greedy_batch(self._h, _ptr(seqs), len(seqs), _ptr(first), n_steps, _ptr(ids),
                                             C.byref(ms)), "cl_decode_greedy_batch")
+        return ids, ms.value
+
+    def decode_sample_batch(self, seqs, first_ids, samplings, first_steps, n_steps: int):
+        """cl_decode_sample_batch: n_steps batched steps, each followed by the device sampler; samplings[b] is greedy or
+        within the device limits.  Returns (ids [n_steps][B], device ms)."""
+        seqs = np.ascontiguousarray(seqs, dtype=np.int32)
+        first = np.ascontiguousarray(first_ids, dtype=np.int32)
+        sps = (Sampling * len(seqs))(*samplings)
+        steps = np.ascontiguousarray(first_steps, dtype=np.uint64)
+        ids = np.empty((n_steps, len(seqs)), np.int32)
+        ms = C.c_float(0)
+        _check(lib().cl_decode_sample_batch(self._h, _ptr(seqs), len(seqs), _ptr(first), sps, _ptr(steps), n_steps, _ptr(ids),
+                                            C.byref(ms)), "cl_decode_sample_batch")
         return ids, ms.value
 
     def decode_step_batch(self, seqs, toks, want_logits: bool = True):
@@ -583,6 +602,28 @@ def op_attn_prefill_variant(q_bf16, k_bf16, v_bf16, n_heads, n_kv, head_dim, var
     _check(lib().cl_op_attn_prefill_variant(device, variant, _ptr(q), _ptr(k), _ptr(v), t, n_heads, n_kv, head_dim, _ptr(out), iters,
                                             C.byref(ms)), "cl_op_attn_prefill_variant")
     return out, (ms.value if iters > 0 else None)
+
+
+def op_sample(logits, samplings, windows, steps, iters=0, device=0):
+    """cl_op_sample: the device sampler on host logits [n_rows][vocab]; windows[r] = row r's history (at most
+    SAMPLE_MAX_WINDOW ids).  Returns (ids [n_rows], mean ms of `iters` timed launches or 0)."""
+    lg = np.ascontiguousarray(logits, dtype=np.float32)
+    n, v = lg.shape
+    win = np.zeros((n, SAMPLE_MAX_WINDOW), np.int32)
+    nwin = np.zeros(n, np.int32)
+    for r, w in enumerate(windows):
+        w = np.asarray(w, np.int32)
+        if w.size > SAMPLE_MAX_WINDOW:
+            raise ValueError(f"window of row {r} holds {w.size} ids (at most {SAMPLE_MAX_WINDOW})")
+        win[r, :w.size] = w
+        nwin[r] = w.size
+    sps = (Sampling * n)(*samplings)
+    st = np.ascontiguousarray(steps, dtype=np.uint64)
+    ids = np.empty(n, np.int32)
+    ms = C.c_float(0)
+    _check(lib().cl_op_sample(device, _ptr(lg), n, v, sps, _ptr(win), _ptr(nwin), _ptr(st), _ptr(ids), iters, C.byref(ms)),
+           "cl_op_sample")
+    return ids, ms.value
 
 
 def op_synth_weights(seed, key, n, scale, device=0):

@@ -109,6 +109,13 @@ typedef struct cl_sampling {
   int32_t ignore_eos;      /* 1 => never stop on EOS (benchmarks) */
 } cl_sampling;
 
+/* Device sampler limits.  A sampled request is drawn on the GPU (no logits copy to the host) when temperature > 0,
+ * 1 <= top_k <= CL_SAMPLE_MAX_TOP_K, top_k < vocab_size, and the repeat penalty is off (repeat_penalty == 1 or
+ * repeat_last_n == 0) or 0 < repeat_last_n <= CL_SAMPLE_MAX_WINDOW.  Every other request is sampled on the host by
+ * cl_sample_token; both draw the same token from the same logits, history and step. */
+#define CL_SAMPLE_MAX_TOP_K 128
+#define CL_SAMPLE_MAX_WINDOW 64
+
 typedef struct cl_result {
   char* text;            /* NUL-terminated UTF-8, malloc'd */
   size_t text_len;
@@ -244,6 +251,14 @@ int cl_decode_greedy(cl_engine* e, cl_seq_t seq, int32_t first_id, int32_t n_ste
 int cl_decode_greedy_batch(cl_engine* e, const cl_seq_t* seqs, int32_t n_seqs,
                            const int32_t* first_ids, int32_t n_steps, int32_t* ids_out,
                            float* device_ms);
+/* Sampled counterpart of cl_decode_greedy_batch: every step runs the batched step, then the device sampler over the
+ * logits of the sequences whose s[b] is sampled (greedy entries keep the step's argmax).  ids_out[i * n_seqs + b] is
+ * what cl_sample_token draws from step i's logits of seqs[b] with s[b], that sequence's whole history (prompt, earlier
+ * tokens, first_ids[b] and the ids drawn before) and step = first_steps[b] + i.  A sampled entry outside the device
+ * limits (CL_SAMPLE_MAX_TOP_K above) returns CL_ERR_INVALID_ARG. */
+int cl_decode_sample_batch(cl_engine* e, const cl_seq_t* seqs, int32_t n_seqs, const int32_t* first_ids,
+                           const cl_sampling* s, const uint64_t* first_steps, int32_t n_steps, int32_t* ids_out,
+                           float* device_ms);
 /* One batched decode step with caller-chosen input tokens (teacher forcing for the parity tests of the batched
  * path): ids[n_seqs]; logits_out (host, may be NULL) receives [n_seqs][vocab_size] fp32; argmax_out (may be NULL)
  * the greedy next ids. */
@@ -308,6 +323,13 @@ int cl_op_attn_prefill(int device, const uint16_t* q, const uint16_t* k, const u
  * 1: tcgen05 kernel (attn_prefill_tc.cu, head_dim 128), -1: what the engine would pick — and an optional timing loop */
 int cl_op_attn_prefill_variant(int device, int variant, const uint16_t* q, const uint16_t* k, const uint16_t* v, int32_t t,
                                int32_t n_heads, int32_t n_kv, int32_t head_dim, float* out, int32_t iters, float* ms);
+/* device sampler: logits [n_rows][vocab] fp32, s[n_rows], windows [n_rows][CL_SAMPLE_MAX_WINDOW] (row r's history: its
+ * first n_window[r] entries), steps[n_rows] -> ids_out[r] == cl_sample_token(logits[r], vocab, &s[r], windows[r],
+ * n_window[r], steps[r]).  Every row must be sampled (temperature > 0) and within the device limits, else
+ * CL_ERR_INVALID_ARG.  iters > 0: also time that many launches over copies of the logits larger than L2 (*ms: mean). */
+int cl_op_sample(int device, const float* logits, int32_t n_rows, int32_t vocab, const cl_sampling* s,
+                 const int32_t* windows, const int32_t* n_window, const uint64_t* steps, int32_t* ids_out, int32_t iters,
+                 float* ms);
 /* synthetic weight generator (device kernel) -> host copy, for known-answer tests */
 int cl_op_synth_weights(int device, uint64_t seed, int32_t tensor_key, int64_t n, float scale,
                         uint16_t* out_bf16);

@@ -1,6 +1,9 @@
 """Scheduler probe: closed-loop clients straight on the C-ABI (no sockets, no gateway), scheduler accounting per run.
 
-    python tools/sched_probe.py [--max-batch 32] [--gen 256] [--prompt 146] [--conc 32,33,64] [--waves 6]
+    python tools/sched_probe.py [--max-batch 32] [--gen 256] [--prompt 146] [--conc 32,33,64] [--waves 6] [--sampling greedy|ollama]
+
+--sampling ollama sends every request with the Ollama defaults (temperature 0.8, top_k 40, top_p 0.9, repeat_penalty 1.1
+over 64 tokens; seed = request index); CL_SCHED_DEVICE_SAMPLE=0/1 in the environment picks the host or the device sampler.
 """
 import argparse
 import sys
@@ -17,14 +20,19 @@ KEYS = ("tokens_generated", "requests_completed", "preemptions", "sched_decode_s
         "sched_prefill_tokens", "sched_prefill_ns")
 
 
-def run(e, conc, n_req, prompt_len, gen, vocab, jitter=0):
+def run(e, conc, n_req, prompt_len, gen, vocab, jitter=0, sampling="greedy"):
     st0 = e.stats()
     sem = threading.Semaphore(conc)
     lat = []
 
     def one(i):
         ids = (np.arange(prompt_len, dtype=np.int64) * 7919 + i * 104729) % (vocab - 1000) + 500
-        sp = eng.greedy(gen + ((i * 37) % (2 * jitter + 1) - jitter if jitter else 0), ignore_eos=True)
+        n = gen + ((i * 37) % (2 * jitter + 1) - jitter if jitter else 0)
+        if sampling == "ollama":
+            sp = eng.ollama_default_sampling(seed=i, max_new_tokens=n)
+            sp.ignore_eos = 1
+        else:
+            sp = eng.greedy(n, ignore_eos=True)
         t0 = time.time()
         e.generate_ids(ids.astype(np.int32), sp)
         lat.append(time.time() - t0)
@@ -42,7 +50,7 @@ def run(e, conc, n_req, prompt_len, gen, vocab, jitter=0):
     st1 = e.stats()
     a = {k: st1[k] - st0[k] for k in KEYS}
     steps = max(a["sched_decode_steps"], 1)
-    print(f"conc {conc:4d} jitter {jitter:3d}: {n_req / dt:6.2f} req/s  p50 {np.median(lat):.3f}s  mean batch {a['tokens_generated'] / steps:5.2f}  decode {a['sched_decode_ns'] / steps * 1e-6:.3f} ms/step "
+    print(f"{sampling:6s} conc {conc:4d} jitter {jitter:3d}: {n_req / dt:6.2f} req/s  p50 {np.median(lat):.3f}s  mean batch {a['tokens_generated'] / steps:5.2f}  decode {a['sched_decode_ns'] / steps * 1e-6:.3f} ms/step "
           f"({a['sched_decode_ns'] * 1e-9:.2f}s)  prefill {a['sched_prefill_ns'] / max(a['sched_prefill_calls'], 1) * 1e-6:.3f} ms/call x {a['sched_prefill_calls']} "
           f"({a['sched_prefill_ns'] * 1e-9:.2f}s)  wall {dt:.2f}s  preempt {a['preemptions']}", flush=True)
 
@@ -56,10 +64,11 @@ if __name__ == "__main__":
     ap.add_argument("--waves", type=int, default=6)
     ap.add_argument("--preset", default="llama3-8b")
     ap.add_argument("--jitter", default="0", help="comma list: max_new = gen +- jitter (desynchronises the requests)")
+    ap.add_argument("--sampling", choices=("greedy", "ollama"), default="greedy")
     a = ap.parse_args()
     with eng.Engine(preset=a.preset, device=0, seed=1234, max_batch=a.max_batch, max_seqs=a.max_batch + 2, start_scheduler=True) as e:
         V = e.cfg["vocab_size"]
-        run(e, a.max_batch, a.max_batch, a.prompt, 32, V)          # warm-up
+        run(e, a.max_batch, a.max_batch, a.prompt, 32, V, sampling=a.sampling)          # warm-up
         for c in [int(x) for x in a.conc.split(",")]:
             for j in [int(x) for x in a.jitter.split(",")]:
-                run(e, c, a.waves * a.max_batch, a.prompt, a.gen, V, j)
+                run(e, c, a.waves * a.max_batch, a.prompt, a.gen, V, j, a.sampling)
