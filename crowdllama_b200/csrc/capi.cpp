@@ -136,6 +136,22 @@ int cl_generate_ids(cl_engine* e, const int32_t* prompt_ids, int32_t n_prompt, c
   CL_GUARD(return e->impl.generate_ids(prompt_ids, n_prompt, sp, out);)
 }
 
+int cl_generate_ids_logprobs(cl_engine* e, const int32_t* prompt_ids, int32_t n_prompt, const cl_sampling* s, int32_t top_n,
+                             cl_result* out, cl_logprobs* lp) {
+  if (!e || !out || !lp || top_n < 0 || top_n > CL_MAX_TOP_LOGPROBS) return CL_ERR_INVALID_ARG;
+  cl_sampling sp;
+  if (s) sp = *s; else cl_default_sampling(&sp);
+  CL_GUARD(return e->impl.generate_ids(prompt_ids, n_prompt, sp, out, nullptr, top_n, lp);)
+}
+
+void cl_logprobs_free(cl_logprobs* l) {
+  if (!l) return;
+  free(l->logprob);
+  free(l->top_ids);
+  free(l->top_logprobs);
+  memset(l, 0, sizeof *l);
+}
+
 namespace {
 // incremental detokeniser: emits only text that later tokens cannot change (an incomplete UTF-8 tail is held back)
 struct StreamText {
@@ -162,7 +178,7 @@ struct StreamText {
   }
 };
 struct TextSinkCtx { StreamText st; cl_token_cb cb; void* user; };
-int text_sink(void* u, const int32_t* ids, int n) {
+int text_sink(void* u, const int32_t* ids, const LogprobRecord*, int n) {
   auto* c = (TextSinkCtx*)u;
   const std::string delta = c->st.feed(ids, n, false);
   return c->cb(c->user, delta.data(), delta.size(), ids, n);
@@ -170,8 +186,10 @@ int text_sink(void* u, const int32_t* ids, int n) {
 int64_t wall_ns() {
   return std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::system_clock::now().time_since_epoch()).count();
 }
-std::vector<uint8_t> response_frame(const std::string& model, const std::string& text, bool done, const std::string& reason) {
+std::vector<uint8_t> response_frame(const std::string& model, const std::string& text, bool done, const std::string& reason,
+                                    std::vector<PbTokenLogprob> logprobs = {}) {
   PbGenerateResponse pr;
+  pr.logprobs = std::move(logprobs);
   pr.model = model;
   const int64_t ns = wall_ns();
   pr.created_at_sec = ns / 1000000000ll;
@@ -183,12 +201,32 @@ std::vector<uint8_t> response_frame(const std::string& model, const std::string&
   pr.total_duration = done ? ns : 0;       // api.go:84: the reference stores time.Now().UnixNano() here
   return pb_encode_response(pr);
 }
-struct FrameSinkCtx { StreamText st; cl_frame_cb cb; void* user; std::string model; };
-int frame_sink(void* u, const int32_t* ids, int n) {
+// GenerateResponse.logprobs entry of one generated id
+PbTokenLogprob token_logprob(const Tokenizer& tok, int32_t id, const LogprobRecord& r, int top_n) {
+  PbTokenLogprob t;
+  t.token = tok.token_bytes(id);
+  t.logprob = r.logprob;
+  for (int j = 0; j < top_n; ++j) {
+    if (r.top_ids[j] < 0) break;                     // a vocabulary smaller than top_n
+    t.top_logprobs.push_back(PbTopLogprob{tok.token_bytes(r.top_ids[j]), r.top_logprobs[j]});
+  }
+  return t;
+}
+// a frame carries the records of the ids its text covers: ids whose bytes are held back (an open UTF-8 sequence) wait
+// for the next frame, the final frame takes whatever is left
+struct FrameSinkCtx {
+  StreamText st; cl_frame_cb cb; void* user; std::string model;
+  int top_n = -1;
+  std::vector<PbTokenLogprob> pending;
+};
+int frame_sink(void* u, const int32_t* ids, const LogprobRecord* lp, int n) {
   auto* c = (FrameSinkCtx*)u;
+  if (lp && c->top_n >= 0)
+    for (int i = 0; i < n; ++i) c->pending.push_back(token_logprob(*c->st.tok, ids[i], lp[i], c->top_n));
   const std::string delta = c->st.feed(ids, n, false);
   if (delta.empty()) return 0;
-  const std::vector<uint8_t> f = response_frame(c->model, delta, false, "");
+  const std::vector<uint8_t> f = response_frame(c->model, delta, false, "", std::move(c->pending));
+  c->pending.clear();
   return c->cb(c->user, f.data(), f.size());
 }
 int check_model(cl_engine* e, const char* model) {
@@ -253,24 +291,43 @@ static int handle_message_impl(cl_engine* e, const uint8_t* req, size_t req_len,
   cl_sampling sp;
   if (s) sp = *s; else cl_default_sampling(&sp);
   apply_options(gr.opt, &sp);                                   // request options win over the worker's defaults
+  // log-probabilities (options fields 9 / 10): top_logprobs alone asks for nothing, as in Ollama
+  int top_n = -1;
+  if (gr.opt.logprobs) {
+    top_n = gr.opt.top_logprobs;
+    if (top_n < 0 || top_n > CL_MAX_TOP_LOGPROBS) {
+      set_last_error("top_logprobs must be within 0.." + std::to_string(CL_MAX_TOP_LOGPROBS));
+      return CL_ERR_INVALID_ARG;
+    }
+  }
   std::vector<int32_t> ids = prompt_ids(e, gr.prompt.data(), gr.prompt.size(), gr.opt.raw);
   cl_result r;
+  cl_logprobs lp{};
   if (gr.stream && allow_stream) {
     // streaming (SURVEY.md §8f row 4): Done=false frames carrying text deltas, then one Done=true frame
-    FrameSinkCtx ctx{StreamText{e->impl.tok.get(), {}, 0}, cb, user, gr.model};
+    FrameSinkCtx ctx{StreamText{e->impl.tok.get(), {}, 0}, cb, user, gr.model, top_n, {}};
     Engine::TokenSink sink{frame_sink, &ctx};
-    const int rc = e->impl.generate_ids(ids.data(), (int)ids.size(), sp, &r, &sink);
+    const int rc = e->impl.generate_ids(ids.data(), (int)ids.size(), sp, &r, &sink, top_n, &lp);
     if (rc) return rc;
     const std::string tail = ctx.st.feed(nullptr, 0, true);
-    const std::vector<uint8_t> f = response_frame(gr.model, tail, true, r.done_reason);
+    const std::vector<uint8_t> f = response_frame(gr.model, tail, true, r.done_reason, std::move(ctx.pending));
     cl_result_free(&r);
+    cl_logprobs_free(&lp);
     cb(user, f.data(), f.size());
     return CL_OK;
   }
-  const int rc = e->impl.generate_ids(ids.data(), (int)ids.size(), sp, &r);
+  const int rc = e->impl.generate_ids(ids.data(), (int)ids.size(), sp, &r, nullptr, top_n, &lp);
   if (rc) return rc;
-  const std::vector<uint8_t> f = response_frame(gr.model, std::string(r.text, r.text_len), true, r.done_reason);
+  std::vector<PbTokenLogprob> entries;
+  for (int i = 0; top_n >= 0 && i < lp.n_tokens; ++i) {
+    LogprobRecord rec;
+    rec.logprob = lp.logprob[i];
+    for (int j = 0; j < lp.top_n; ++j) { rec.top_ids[j] = lp.top_ids[i * lp.top_n + j]; rec.top_logprobs[j] = lp.top_logprobs[i * lp.top_n + j]; }
+    entries.push_back(token_logprob(*e->impl.tok, r.token_ids[i], rec, lp.top_n));
+  }
+  const std::vector<uint8_t> f = response_frame(gr.model, std::string(r.text, r.text_len), true, r.done_reason, std::move(entries));
   cl_result_free(&r);
+  cl_logprobs_free(&lp);
   cb(user, f.data(), f.size());
   return CL_OK;
 }

@@ -36,6 +36,8 @@ Engine::~Engine() {
   for (void* p : allocs_) cudaFree(p);
   if (h_logits_pinned_) cudaFreeHost(h_logits_pinned_);
   if (h_ids_pinned_) cudaFreeHost(h_ids_pinned_);
+  if (h_lp_rec_) cudaFreeHost(h_lp_rec_);
+  if (h_lp_ring_) cudaFreeHost(h_lp_ring_);
   if (ev0_) cudaEventDestroy(ev0_);
   if (ev1_) cudaEventDestroy(ev1_);
   if (stream_) cudaStreamDestroy(stream_);
@@ -820,14 +822,25 @@ int Engine::prefill(cl_seq_t s, const int32_t* ids, int n, float* logits_out) {
   return prefill_tokenwise(s, ids, n, logits_out);
 }
 
-int Engine::decode_greedy(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms) {
-  return decode_loop(ss, B, first_ids, n_steps, ids_out, device_ms, false);
+int Engine::decode_greedy(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms,
+                          const int* top_n, LogprobRecord* lp_out) {
+  return decode_loop(ss, B, first_ids, n_steps, ids_out, device_ms, false, top_n, lp_out);
 }
 
-// n_steps batched steps on the device; with `sample`, the sampler runs after every step (slots set up by sample_setup)
+// n_steps batched steps on the device; with `sample`, the sampler runs after every step (slots set up by sample_setup);
+// with a top_n >= 0 in top_n[0..B) (and lp_out), logprobs_kernel runs after that over all B rows (the largest top_n)
 int Engine::decode_loop(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms,
-                        bool sample) {
+                        bool sample, const int* top_n, LogprobRecord* lp_out) {
   if (B <= 0 || B > max_batch_ || n_steps <= 0) { set_last_error("bad batch / steps"); return CL_ERR_INVALID_ARG; }
+  int lp_n = -1;
+  for (int b = 0; top_n && lp_out && b < B; ++b) {
+    if (top_n[b] > CL_MAX_TOP_LOGPROBS) { set_last_error("top_n above CL_MAX_TOP_LOGPROBS"); return CL_ERR_INVALID_ARG; }
+    lp_n = std::max(lp_n, top_n[b]);
+  }
+  if (lp_n >= 0) {
+    const int rc = ensure_logprobs();
+    if (rc) return rc;
+  }
   for (int b = 0; b < B; ++b) {
     const int s = ss[b];
     if (s < 0 || s >= max_seqs_ || !seqs_[s].live) return CL_ERR_BAD_SEQ;
@@ -852,16 +865,21 @@ int Engine::decode_loop(const cl_seq_t* ss, int B, const int32_t* first_ids, int
     for (int i = 0; i < chunk; ++i) {
       int rc = run_step_graph(B);
       if (rc == CL_OK && sample) rc = launch_sampler(B, d_slots_, true);
+      if (rc == CL_OK && lp_n >= 0) rc = launch_logprobs(B, d_slots_, true, lp_n);
       if (rc) return rc;
     }
     CL_CUDA_OK(cudaEventRecord(ev1_, stream_));
     CL_CUDA_OK(cudaMemcpyAsync(h_ids_pinned_, d_ids_ring_, (size_t)chunk * max_batch_ * 4, cudaMemcpyDeviceToHost, stream_));
+    if (lp_n >= 0)   // the B entries of each ring row
+      CL_CUDA_OK(cudaMemcpy2DAsync(h_lp_ring_, (size_t)B * sizeof(LogprobRecord), d_lp_ring_, (size_t)max_batch_ * sizeof(LogprobRecord),
+                                   (size_t)B * sizeof(LogprobRecord), (size_t)chunk, cudaMemcpyDeviceToHost, stream_));
     CL_CUDA_OK(cudaStreamSynchronize(stream_));
     float ms = 0.f;
     CL_CUDA_OK(cudaEventElapsedTime(&ms, ev0_, ev1_));
     total_ms += ms;
     for (int i = 0; i < chunk; ++i)
       for (int b = 0; b < B; ++b) ids_out[(size_t)(done + i) * B + b] = h_ids_pinned_[(size_t)i * max_batch_ + b];
+    if (lp_n >= 0) memcpy(lp_out + (size_t)done * B, h_lp_ring_, (size_t)chunk * B * sizeof(LogprobRecord));
     done += chunk;
   }
   for (int b = 0; b < B; ++b) {
@@ -930,7 +948,7 @@ int Engine::sample_slots(const cl_seq_t* ss, int n, int32_t* ids_out) {
 }
 
 int Engine::decode_sample(const cl_seq_t* ss, int B, const int32_t* first_ids, const cl_sampling* sps, const uint64_t* first_steps,
-                          int n_steps, int32_t* ids_out, float* device_ms) {
+                          int n_steps, int32_t* ids_out, float* device_ms, const int* top_n, LogprobRecord* lp_out) {
   if (B <= 0 || B > max_batch_ || n_steps <= 0) { set_last_error("bad batch / steps"); return CL_ERR_INVALID_ARG; }
   if (!d_sample_state_) { set_last_error("vocabulary too large for the device sampler"); return CL_ERR_INVALID_ARG; }
   bool any = false;
@@ -953,7 +971,63 @@ int Engine::decode_sample(const cl_seq_t* ss, int B, const int32_t* first_ids, c
     const int rc = sample_setup(ss[b], sps[b], hist.data(), (int)hist.size(), first_steps[b]);
     if (rc) return rc;
   }
-  return decode_loop(ss, B, first_ids, n_steps, ids_out, device_ms, any);
+  return decode_loop(ss, B, first_ids, n_steps, ids_out, device_ms, any, top_n, lp_out);
+}
+
+// ---- log-probabilities (logprobs_kernel in sample_kernels.cu) ----------------------------------------
+// Allocated by the first request that asks: an engine that never sees one holds none of it (the ring alone is 21 MB at
+// max_batch 128).
+int Engine::ensure_logprobs() {
+  if (d_lp_rec_) return CL_OK;
+  const int nblk = logprob_blocks(cfg.vocab_size);
+  if (!nblk) { set_last_error("vocabulary too large for logprobs_kernel"); return CL_ERR_INVALID_ARG; }
+  const size_t S = (size_t)max_seqs_, ring = (size_t)ring_steps_ * max_batch_;
+  DMALLOC(d_lp_ring_, ring * sizeof(LogprobRecord));
+  DMALLOC(d_lp_part_, S * nblk * CL_MAX_TOP_LOGPROBS * sizeof(unsigned long long));
+  DMALLOC(d_lp_stat_, S * nblk * sizeof(float2));
+  DMALLOC(d_lp_cnt_, S * 4);
+  DMALLOC(d_lp_slots_, S * 4);
+  CL_CUDA_OK(cudaMemsetAsync(d_lp_cnt_, 0, S * 4, stream_));
+  CL_CUDA_OK(cudaMallocHost(&h_lp_rec_, S * sizeof(LogprobRecord)));
+  CL_CUDA_OK(cudaMallocHost(&h_lp_ring_, ring * sizeof(LogprobRecord)));
+  DMALLOC(d_lp_rec_, S * sizeof(LogprobRecord));   // last: its presence marks the set-up as complete
+  return CL_OK;
+}
+
+int Engine::launch_logprobs(int B, const int* d_slots, bool ring, int top_n) {
+  LogprobArgs a;
+  a.logits = d_logits_; a.vocab = cfg.vocab_size; a.tok = d_tok_; a.rec = d_lp_rec_;
+  if (ring) { a.rec_ring = d_lp_ring_; a.step_counter = d_step_counter_; a.ring_steps = ring_steps_; a.ring_stride = max_batch_; }
+  a.part = d_lp_part_; a.stat = d_lp_stat_; a.counters = d_lp_cnt_; a.slots = d_slots; a.batch = B;
+  a.nblk = logprob_blocks(cfg.vocab_size); a.top_n = top_n;
+  const int n = ::cl::launch_logprobs(a, stream_);
+  if (n < 0) { set_last_error(std::string("launch_logprobs: ") + cudaGetErrorString(cudaGetLastError())); return CL_ERR_CUDA; }
+  launches_ += n;
+  return CL_OK;
+}
+
+int Engine::logprobs_enqueue(const cl_seq_t* ss, int n, int top_n) {
+  if (n <= 0) return CL_OK;
+  if (n > max_seqs_ || top_n < 0 || top_n > CL_MAX_TOP_LOGPROBS) { set_last_error("logprobs_enqueue: bad slot list"); return CL_ERR_INVALID_ARG; }
+  int rc = ensure_logprobs();
+  if (rc) return rc;
+  if (lp_last_slots_.size() != (size_t)n || !std::equal(ss, ss + n, lp_last_slots_.begin())) {   // steady batches upload nothing
+    lp_last_slots_.assign(ss, ss + n);
+    CL_CUDA_OK(cudaMemcpyAsync(d_lp_slots_, lp_last_slots_.data(), (size_t)n * 4, cudaMemcpyHostToDevice, stream_));
+  }
+  rc = launch_logprobs(n, d_lp_slots_, false, top_n);
+  if (rc) return rc;
+  const int lo = *std::min_element(ss, ss + n), hi = *std::max_element(ss, ss + n);
+  CL_CUDA_OK(cudaMemcpyAsync(h_lp_rec_ + lo, d_lp_rec_ + lo, (size_t)(hi - lo + 1) * sizeof(LogprobRecord), cudaMemcpyDeviceToHost, stream_));
+  return CL_OK;
+}
+
+int Engine::logprobs_read(const cl_seq_t* ss, int n, int top_n, LogprobRecord* out) {
+  const int rc = logprobs_enqueue(ss, n, top_n);
+  if (rc) return rc;
+  CL_CUDA_OK(cudaStreamSynchronize(stream_));
+  for (int i = 0; i < n; ++i) out[i] = h_lp_rec_[ss[i]];
+  return CL_OK;
 }
 
 // ---- parity / benchmark aids ------------------------------------------------------------------------

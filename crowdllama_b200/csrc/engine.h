@@ -73,6 +73,8 @@ class Tokenizer {
   // chat framing the Ollama server applies upstream of the model (role forced to "user", api.go:111-116)
   virtual std::string apply_chat_template(const std::string& user_prompt) const = 0;
   virtual int vocab_size() const = 0;
+  // the surface bytes of one id on its own (log-probability entries); special tokens give their content
+  virtual std::string token_bytes(int id) const { return decode_bytes({id}); }
 };
 
 // byte-level fallback (no vocab files exist offline; SURVEY.md §8f row 2): ids 0..2 = <pad>, <bos>, <eos>;
@@ -113,14 +115,18 @@ struct PbGenerateOptions {
   uint32_t has = 0;   // bit i set <=> field number i present
   uint64_t seed = 0; float temperature = 0.f; int32_t top_k = 0; float top_p = 0.f; float repeat_penalty = 0.f;
   int32_t repeat_last_n = 0; int32_t num_predict = 0; bool raw = false;
+  bool logprobs = false; int32_t top_logprobs = 0;   // fields 9, 10
 };
 struct PbGenerateRequest { std::string model, prompt; bool stream = false; PbGenerateOptions opt; };
 // request options override the caller's default sampling field by field
 void apply_options(const PbGenerateOptions& o, cl_sampling* sp);
+struct PbTopLogprob { std::string token; float logprob = 0.f; };
+struct PbTokenLogprob { std::string token; float logprob = 0.f; std::vector<PbTopLogprob> top_logprobs; };
 struct PbGenerateResponse {
   std::string model, response, done_reason, worker_id;
   int64_t created_at_sec = 0; int32_t created_at_nanos = 0;
   bool done = false; int64_t total_duration = 0;
+  std::vector<PbTokenLogprob> logprobs;               // field 8: one per token id the frame covers
 };
 bool pb_decode_request(const uint8_t* data, size_t len, PbGenerateRequest* out);  // false: not a GenerateRequest
 std::vector<uint8_t> pb_encode_response(const PbGenerateResponse& r);
@@ -156,11 +162,13 @@ class Engine {
   // several prompts in one pass of the tile path (prefill.cu); logits_out: [n_seqs][vocab] or nullptr
   int prefill_multi(int n_seqs, const cl_seq_t* ss, const int32_t* const* ids, const int* lens, float* logits_out);
   int decode_step(cl_seq_t s, int32_t id, float* logits_out, int32_t* argmax_out);
+  // top_n (optional, [n_seqs], -1: not asked): logprobs_kernel after every step; lp_out[i * n_seqs + b] receives the
+  // record of ids_out[i * n_seqs + b] (rows that did not ask: unspecified)
   int decode_greedy(const cl_seq_t* seqs, int n_seqs, const int32_t* first_ids, int n_steps, int32_t* ids_out,
-                    float* device_ms);
+                    float* device_ms, const int* top_n = nullptr, LogprobRecord* lp_out = nullptr);
   // sampled counterpart: step graph + device sampler per step; sps[b] greedy or within the device limits
   int decode_sample(const cl_seq_t* seqs, int n_seqs, const int32_t* first_ids, const cl_sampling* sps, const uint64_t* first_steps,
-                    int n_steps, int32_t* ids_out, float* device_ms);
+                    int n_steps, int32_t* ids_out, float* device_ms, const int* top_n = nullptr, LogprobRecord* lp_out = nullptr);
   // device sampler (sample_kernels.cu): true if the request's options fit its limits (clengine.h CL_SAMPLE_MAX_*)
   static bool sample_qualifies(const cl_sampling& sp, int vocab);
   // the sampler state of one slot (top_k 0: not sampled on the device); window = the last repeat_last_n ids of hist
@@ -171,6 +179,13 @@ class Engine {
   // draw the next token of the n slots whose last-position logits an admission has just left in d_logits_
   // (d_tok_[slot] is overwritten); ids_out (host, may be nullptr) receives them
   int sample_slots(const cl_seq_t* ss, int n, int32_t* ids_out);
+  // log-probabilities (logprobs_kernel): enqueue one launch over the n slots whose logits rows a step or an admission has
+  // just left in d_logits_ (the emitted id read from d_tok_[slot]) and the copy of their records to the host; after the
+  // next synchronisation of the stream, lp_host(slot) holds them.  The buffers are allocated on the first call.
+  int logprobs_enqueue(const cl_seq_t* ss, int n, int top_n);
+  const LogprobRecord& lp_host(cl_seq_t s) const { return h_lp_rec_[s]; }
+  // logprobs_enqueue, then wait for the stream: out[i] = the record of ss[i]
+  int logprobs_read(const cl_seq_t* ss, int n, int top_n, LogprobRecord* out);
   int set_tensor(int layer, int kind, const uint16_t* data, int64_t n);
   int load_safetensors(const std::string& path);   // HF llama-layout checkpoint (file or directory) -> set_tensor (weights_io.cpp)
   // parity / benchmark aids (token level)
@@ -184,8 +199,11 @@ class Engine {
 
   // request-level (scheduler.cpp)
   // sink (optional): called on the CALLING thread with every batch of newly generated ids; nonzero return cancels
-  struct TokenSink { int (*fn)(void* user, const int32_t* ids, int n) = nullptr; void* user = nullptr; };
-  int generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling& sp, cl_result* out, const TokenSink* sink = nullptr);
+  // lp: the log-probability records of the ids (nullptr unless the request asked for them)
+  struct TokenSink { int (*fn)(void* user, const int32_t* ids, const LogprobRecord* lp, int n) = nullptr; void* user = nullptr; };
+  // top_n >= 0: the log-probabilities of every generated token with top_n alternatives go to lp_out (and the sink)
+  int generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling& sp, cl_result* out, const TokenSink* sink = nullptr,
+                   int top_n = -1, cl_logprobs* lp_out = nullptr);
   void scheduler_main();
   void start_scheduler();
   void stop_scheduler();
@@ -208,7 +226,11 @@ class Engine {
   void precapture_graphs();                       // graph launch (or eager enqueue)
   int read_logits(int slot, float* out);
   int launch_sampler(int B, const int* d_slots, bool ring);   // sampler over d_slots[0..B) (ring: write the step's ids_ring row)
-  int decode_loop(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms, bool sample);
+  // logprobs_kernel over d_slots[0..B) (ring: write the step's record ring row, else the per-slot records)
+  int launch_logprobs(int B, const int* d_slots, bool ring, int top_n);
+  int ensure_logprobs();                                      // lazy allocation of the record buffers
+  int decode_loop(const cl_seq_t* ss, int B, const int32_t* first_ids, int n_steps, int32_t* ids_out, float* device_ms, bool sample,
+                  const int* top_n, LogprobRecord* lp_out);
   int prefill_tokenwise(cl_seq_t s, const int32_t* ids, int n, float* logits_out);
   int prefill_chunked(cl_seq_t s, const int32_t* ids, int n, float* logits_out);
   int ensure_prefill_ws(int tokens);  // tcgen05 path (prefill.cu)
@@ -261,6 +283,16 @@ class Engine {
   unsigned* d_sample_cnt_ = nullptr;                     // [max_seqs]
   int* d_sample_slots_ = nullptr;                        // [max_seqs] slot list of an admission's sampler launch
   int sample_nblk_ = 0;                                  // 0: vocabulary too large for the device sampler
+  // log-probabilities (logprobs_kernel), allocated by the first request that asks
+  LogprobRecord* d_lp_rec_ = nullptr;                    // [max_seqs]
+  LogprobRecord* d_lp_ring_ = nullptr;                   // [ring_steps][max_batch]
+  LogprobRecord* h_lp_rec_ = nullptr;                    // pinned [max_seqs]
+  LogprobRecord* h_lp_ring_ = nullptr;                   // pinned [ring_steps][max_batch]
+  unsigned long long* d_lp_part_ = nullptr;              // [max_seqs][nblk][CL_MAX_TOP_LOGPROBS]
+  float2* d_lp_stat_ = nullptr;                          // [max_seqs][nblk]
+  unsigned* d_lp_cnt_ = nullptr;                         // [max_seqs]
+  int* d_lp_slots_ = nullptr;                            // [max_seqs] slot list of the last logprobs_enqueue
+  std::vector<int> lp_last_slots_;                       // what d_lp_slots_ holds
 
   // prefill workspace (allocated lazily)
   struct PrefillWs {

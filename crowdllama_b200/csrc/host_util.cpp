@@ -171,15 +171,20 @@ int32_t sample_token(const float* logits, int32_t vocab, const cl_sampling& sp, 
 //                      GenerateOptions options = 4; }                       <- EXTENSION (SURVEY.md §8f row 3)
 //   GenerateOptions  { optional uint64 seed = 1; optional float temperature = 2; optional int32 top_k = 3;
 //                      optional float top_p = 4; optional float repeat_penalty = 5;
-//                      optional int32 repeat_last_n = 6; optional int32 num_predict = 7; optional bool raw = 8; }
+//                      optional int32 repeat_last_n = 6; optional int32 num_predict = 7; optional bool raw = 8;
+//                      optional bool logprobs = 9; optional int32 top_logprobs = 10; }        <- EXTENSION
 //   GenerateResponse { string model = 1; google.protobuf.Timestamp created_at = 2;
 //                      string response = 3; bool done = 4; string done_reason = 5;
-//                      string worker_id = 6; int64 total_duration = 7; }
+//                      string worker_id = 6; int64 total_duration = 7;
+//                      repeated TokenLogprob logprobs = 8; }                                 <- EXTENSION
+//   TokenLogprob     { bytes token = 1; float logprob = 2; repeated TopLogprob top_logprobs = 3; }
+//   TopLogprob       { bytes token = 1; float logprob = 2; }
 // ================================================================================================
 enum { kReqOptions = 4, kOptSeed = 1, kOptTemperature = 2, kOptTopK = 3, kOptTopP = 4, kOptRepeatPenalty = 5, kOptRepeatLastN = 6,
-       kOptNumPredict = 7, kOptRaw = 8 };
+       kOptNumPredict = 7, kOptRaw = 8, kOptLogprobs = 9, kOptTopLogprobs = 10 };
 enum { kBaseReq = 1, kBaseResp = 2, kReqModel = 1, kReqPrompt = 2, kReqStream = 3, kRespModel = 1, kRespCreated = 2,
-       kRespResponse = 3, kRespDone = 4, kRespDoneReason = 5, kRespWorkerId = 6, kRespTotalDuration = 7 };
+       kRespResponse = 3, kRespDone = 4, kRespDoneReason = 5, kRespWorkerId = 6, kRespTotalDuration = 7, kRespLogprobs = 8,
+       kLpToken = 1, kLpLogprob = 2, kLpTop = 3 };
 
 static bool rd_varint(const uint8_t*& p, const uint8_t* end, uint64_t* v) {
   uint64_t r = 0;
@@ -205,13 +210,16 @@ static bool decode_options(const uint8_t* q, const uint8_t* qe, PbGenerateOption
     uint64_t k;
     if (!rd_varint(q, qe, &k)) return false;
     const int f = (int)(k >> 3), wt = (int)(k & 7);
-    if (wt == 0 && (f == kOptSeed || f == kOptTopK || f == kOptRepeatLastN || f == kOptNumPredict || f == kOptRaw)) {
+    if (wt == 0 && (f == kOptSeed || f == kOptTopK || f == kOptRepeatLastN || f == kOptNumPredict || f == kOptRaw || f == kOptLogprobs ||
+                    f == kOptTopLogprobs)) {
       uint64_t v;
       if (!rd_varint(q, qe, &v)) return false;
       if (f == kOptSeed) o->seed = v;
       else if (f == kOptTopK) o->top_k = (int32_t)(int64_t)v;
       else if (f == kOptRepeatLastN) o->repeat_last_n = (int32_t)(int64_t)v;
       else if (f == kOptNumPredict) o->num_predict = (int32_t)(int64_t)v;
+      else if (f == kOptLogprobs) o->logprobs = v != 0;
+      else if (f == kOptTopLogprobs) o->top_logprobs = (int32_t)(int64_t)v;
       else o->raw = v != 0;
       o->has |= 1u << f;
     } else if (wt == 5 && (f == kOptTemperature || f == kOptTopP || f == kOptRepeatPenalty)) {
@@ -287,6 +295,18 @@ static void wr_i64(std::vector<uint8_t>& b, int field, int64_t v) {
   wr_varint(b, (uint64_t)field << 3 | 0);
   wr_varint(b, (uint64_t)v);
 }
+static void wr_f32(std::vector<uint8_t>& b, int field, float v) {
+  if (v == 0.f) return;
+  wr_varint(b, (uint64_t)field << 3 | 5);
+  uint8_t x[4];
+  memcpy(x, &v, 4);
+  b.insert(b.end(), x, x + 4);
+}
+static void wr_msg(std::vector<uint8_t>& b, int field, const std::vector<uint8_t>& m) {   // present even when empty
+  wr_varint(b, (uint64_t)field << 3 | 2);
+  wr_varint(b, m.size());
+  b.insert(b.end(), m.begin(), m.end());
+}
 std::vector<uint8_t> pb_encode_response(const PbGenerateResponse& r) {
   std::vector<uint8_t> ts;
   wr_i64(ts, 1, r.created_at_sec);
@@ -303,6 +323,18 @@ std::vector<uint8_t> pb_encode_response(const PbGenerateResponse& r) {
   wr_str(in, kRespDoneReason, r.done_reason);
   wr_str(in, kRespWorkerId, r.worker_id);
   wr_i64(in, kRespTotalDuration, r.total_duration);
+  for (const auto& t : r.logprobs) {
+    std::vector<uint8_t> m;
+    wr_str(m, kLpToken, t.token);
+    wr_f32(m, kLpLogprob, t.logprob);
+    for (const auto& a : t.top_logprobs) {
+      std::vector<uint8_t> n;
+      wr_str(n, kLpToken, a.token);
+      wr_f32(n, kLpLogprob, a.logprob);
+      wr_msg(m, kLpTop, n);
+    }
+    wr_msg(in, kRespLogprobs, m);
+  }
   std::vector<uint8_t> out;
   wr_varint(out, (uint64_t)kBaseResp << 3 | 2);
   wr_varint(out, in.size());

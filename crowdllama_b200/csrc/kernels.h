@@ -129,6 +129,33 @@ constexpr int kSampleCand = CL_SAMPLE_MAX_TOP_K + CL_SAMPLE_MAX_WINDOW;   // can
 int sample_blocks(int vocab);        // CTAs per row; 0 if the vocabulary is too large for the sampler
 int launch_sample(const SampleArgs& a, cudaStream_t st);
 
+// one generated token's log-probabilities (logprobs_kernel in sample_kernels.cu; clengine.h cl_logprobs)
+struct LogprobRecord {
+  float lse = 0.f;                                  // logsumexp of the row
+  float logprob = 0.f;                              // logits[chosen] - lse
+  int top_ids[CL_MAX_TOP_LOGPROBS] = {};            // [0, top_n): value descending, then id ascending
+  float top_logprobs[CL_MAX_TOP_LOGPROBS] = {};
+};
+
+struct LogprobArgs {
+  const float* logits = nullptr;     // [slot][vocab], read in place
+  int vocab = 0;
+  const int* tok = nullptr;          // [slot] the emitted id of the row (step tail's argmax or the device sampler's draw)
+  LogprobRecord* rec = nullptr;      // [slot] (used when rec_ring is nullptr)
+  LogprobRecord* rec_ring = nullptr; // [ring_steps][ring_stride]: entry b of the step just run (as SampleArgs::ids_ring)
+  const int* step_counter = nullptr;
+  int ring_steps = 0, ring_stride = 0;
+  unsigned long long* part = nullptr;// [slot][nblk][CL_MAX_TOP_LOGPROBS] per-CTA top keys
+  float2* stat = nullptr;            // [slot][nblk] per-CTA (max, sum of exp(x - max))
+  unsigned* counters = nullptr;      // [slot] arrival counters (self re-arming)
+  const int* slots = nullptr;        // [batch] (nullptr: identity)
+  int batch = 1;
+  int nblk = 1;                      // CTAs per row: logprob_blocks(vocab)
+  int top_n = 0;                     // 0..CL_MAX_TOP_LOGPROBS, the same for every row of the launch
+};
+int logprob_blocks(int vocab);       // CTAs per row; 0 if the vocabulary is too large
+int launch_logprobs(const LogprobArgs& a, cudaStream_t st);
+
 // every launcher returns the number of kernels it enqueued (for cl_stats.kernel_launches)
 int launch_gemv(int variant, int epi, bool norm, const GemvArgs& a, cudaStream_t st, bool pdl, int* n_ctas = nullptr);
 int launch_attn_decode(const AttnDecodeArgs& a, cudaStream_t st, bool pdl);

@@ -275,6 +275,67 @@ int cl_op_sample(int device, const float* logits, int32_t n_rows, int32_t vocab,
   return CL_OK;
 }
 
+int cl_op_logprobs(int device, const float* logits, int32_t n_rows, int32_t vocab, const int32_t* chosen, int32_t top_n,
+                   float* logprob, int32_t* top_ids, float* top_logprobs, int32_t iters, float* ms) {
+  if (!logits || !chosen || !logprob || n_rows <= 0 || vocab <= 0 || top_n < 0 || top_n > CL_MAX_TOP_LOGPROBS ||
+      (top_n > 0 && (!top_ids || !top_logprobs)))
+    return CL_ERR_INVALID_ARG;
+  int rc = check_device(device);
+  if (rc) return rc;
+  const int nblk = logprob_blocks(vocab);
+  if (!nblk) { set_last_error("vocabulary too large for logprobs_kernel"); return CL_ERR_INVALID_ARG; }
+  const size_t row_bytes = (size_t)vocab * 4, bytes = (size_t)n_rows * row_bytes;
+  DevBuf dl, dtok, drec, dpart, dstat, dcnt;
+  CL_CUDA_OK(dl.upload(logits, bytes));
+  CL_CUDA_OK(dtok.upload(chosen, (size_t)n_rows * 4));
+  CL_CUDA_OK(drec.alloc((size_t)n_rows * sizeof(LogprobRecord)));
+  CL_CUDA_OK(dpart.alloc((size_t)n_rows * nblk * CL_MAX_TOP_LOGPROBS * sizeof(unsigned long long)));
+  CL_CUDA_OK(dstat.alloc((size_t)n_rows * nblk * sizeof(float2)));
+  CL_CUDA_OK(dcnt.alloc((size_t)n_rows * 4));
+  CL_CUDA_OK(cudaMemset(dcnt.p, 0, (size_t)n_rows * 4));
+  LogprobArgs a;
+  a.logits = dl.as<float>(); a.vocab = vocab; a.tok = dtok.as<int>(); a.rec = drec.as<LogprobRecord>();
+  a.part = dpart.as<unsigned long long>(); a.stat = dstat.as<float2>(); a.counters = dcnt.as<unsigned>();
+  a.batch = n_rows; a.nblk = nblk; a.top_n = top_n;
+  if (launch_logprobs(a, nullptr) < 0) { set_last_error(std::string("launch_logprobs: ") + cudaGetErrorString(cudaGetLastError())); return CL_ERR_CUDA; }
+  CL_CUDA_OK(cudaDeviceSynchronize());
+  std::vector<LogprobRecord> rec((size_t)n_rows);
+  CL_CUDA_OK(cudaMemcpy(rec.data(), drec.p, rec.size() * sizeof(LogprobRecord), cudaMemcpyDeviceToHost));
+  for (int r = 0; r < n_rows; ++r) {
+    logprob[r] = rec[r].logprob;
+    for (int j = 0; j < top_n; ++j) {
+      top_ids[(size_t)r * top_n + j] = rec[r].top_ids[j];
+      top_logprobs[(size_t)r * top_n + j] = rec[r].top_logprobs[j];
+    }
+  }
+  if (iters > 0 && ms) {
+    // timing loop over enough copies of the logits to exceed the 126 MB L2 (each launch reads rows no earlier launch left there)
+    const int copies = (int)std::min<size_t>(16, (256ull << 20) / bytes + 1);
+    std::vector<DevBuf> extra(copies > 1 ? copies - 1 : 0);
+    std::vector<const float*> ls{dl.as<float>()};
+    for (auto& b : extra) {
+      CL_CUDA_OK(b.alloc(bytes));
+      CL_CUDA_OK(cudaMemcpy(b.p, dl.p, bytes, cudaMemcpyDeviceToDevice));
+      ls.push_back(b.as<float>());
+    }
+    cudaEvent_t e0, e1;
+    CL_CUDA_OK(cudaEventCreate(&e0));
+    CL_CUDA_OK(cudaEventCreate(&e1));
+    for (int i = 0; i < 3; ++i) { a.logits = ls[i % ls.size()]; launch_logprobs(a, nullptr); }
+    CL_CUDA_OK(cudaDeviceSynchronize());
+    CL_CUDA_OK(cudaEventRecord(e0, nullptr));
+    for (int i = 0; i < iters; ++i) { a.logits = ls[i % ls.size()]; launch_logprobs(a, nullptr); }
+    CL_CUDA_OK(cudaEventRecord(e1, nullptr));
+    CL_CUDA_OK(cudaDeviceSynchronize());
+    float t = 0.f;
+    CL_CUDA_OK(cudaEventElapsedTime(&t, e0, e1));
+    *ms = t / (float)iters;
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+  }
+  return CL_OK;
+}
+
 int cl_op_synth_weights(int device, uint64_t seed, int32_t tensor_key, int64_t n, float scale, uint16_t* out_bf16) {
   if (!out_bf16 || n <= 0) return CL_ERR_INVALID_ARG;
   int rc = check_device(device);

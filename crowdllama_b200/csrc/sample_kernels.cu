@@ -260,6 +260,134 @@ __global__ void __launch_bounds__(kSampleThreads, 1) sample_topk_kernel(const Sa
   }
 }
 
+// ---- log-probabilities of the emitted tokens ----------------------------------------------------------------------
+// Raw distribution: log_softmax of the row as the step left it.  grid (nblk, batch) over the same slices as the sampler;
+// each CTA computes its slice's max m_b and s_b = sum exp(x - m_b) (per-thread sums in a fixed order, then fixed
+// shuffle and shared-memory trees: no float atomics) and, with top_n > 0, the top_n best keys of the slice
+// (top_m_sorted).  The last CTA of the row to arrive merges in block order: M = max m_b, S = sum_b s_b exp(m_b - M),
+// lse = M + log S, and the top_n best of the nblk lists.  A row's record depends only on the row: the same bits at any
+// batch size or position.  -inf entries add nothing to S and rank below every finite entry.
+__global__ void __launch_bounds__(kSampleThreads, 1) logprobs_kernel(const LogprobArgs a) {
+  extern __shared__ unsigned long long sk[];          // kSampleChunk keys (top_n > 0 only)
+  __shared__ float red[32];
+  __shared__ float lse_s;
+  __shared__ int is_last_s;
+  __shared__ SelectShared sel;
+  const int b = blockIdx.y, blk = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int slot = a.slots ? a.slots[b] : b;
+  const int V = a.vocab, nblk = a.nblk, N = a.top_n;
+  const float* lg = a.logits + (size_t)slot * V;
+
+  // ---- 1. slice max, sum of exp(x - max), top_n keys
+  const int C = (V + nblk - 1) / nblk, i0 = blk * C, i1 = min(V, i0 + C);
+  float v[kSamplePerThread];
+  float m = -INFINITY;
+#pragma unroll
+  for (int q = 0; q < kSamplePerThread; ++q) {
+    const int id = i0 + q * kSampleThreads + tid;
+    v[q] = id < i1 ? __ldcs(lg + id) : -INFINITY;
+    m = fmaxf(m, v[q]);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if (lane == 0) red[warp] = m;
+  __syncthreads();
+  m = red[lane];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  __syncthreads();                                     // red[] is reused for the sums
+  float s = 0.f;
+#pragma unroll
+  for (int q = 0; q < kSamplePerThread; ++q) s += v[q] > -INFINITY ? expf(v[q] - m) : 0.f;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) red[warp] = s;
+  __syncthreads();
+  s = red[lane];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  unsigned long long kv[kSamplePerThread];
+  if (N > 0) {
+#pragma unroll
+    for (int q = 0; q < kSamplePerThread; ++q) {
+      const int id = i0 + q * kSampleThreads + tid;
+      kv[q] = id < i1 ? make_key(v[q], id) : 0ull;
+    }
+    top_m_sorted(kv, N, sk, sel);
+  }
+  if (nblk > 1) {
+    unsigned long long* part = a.part + (size_t)slot * nblk * CL_MAX_TOP_LOGPROBS;
+    if (tid < N) part[(size_t)blk * CL_MAX_TOP_LOGPROBS + tid] = sk[tid];
+    if (tid == 0) a.stat[(size_t)slot * nblk + blk] = make_float2(m, s);
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) {
+      const unsigned old = atomicAdd(a.counters + slot, 1u);
+      is_last_s = old == (unsigned)nblk - 1;
+      if (is_last_s) a.counters[slot] = 0u;
+    }
+    __syncthreads();
+    if (!is_last_s) return;
+    __threadfence();
+    // ---- 2. merge in block order (the result does not depend on the arrival order)
+    if (tid == 0) {
+      const float2* st = a.stat + (size_t)slot * nblk;
+      float M = -INFINITY;
+      for (int j = 0; j < nblk; ++j) M = fmaxf(M, __ldcg(&st[j].x));
+      float S = 0.f;
+      for (int j = 0; j < nblk; ++j) {
+        const float2 ms = __ldcg(st + j);
+        if (ms.x > -INFINITY) S += ms.y * expf(ms.x - M);
+      }
+      lse_s = M + logf(S);
+    }
+    if (N > 0) {
+#pragma unroll
+      for (int q = 0; q < kSamplePerThread; ++q) {
+        const int i = q * kSampleThreads + tid;
+        kv[q] = i < nblk * N ? __ldcg(part + (size_t)(i / N) * CL_MAX_TOP_LOGPROBS + i % N) : 0ull;
+      }
+      top_m_sorted(kv, N, sk, sel);                    // ends with __syncthreads: lse_s is visible
+    }
+  } else if (tid == 0) {
+    lse_s = m + logf(s);
+  }
+  __syncthreads();
+
+  // ---- 3. the record
+  const float lse = lse_s;
+  LogprobRecord* r = a.rec_ring ? a.rec_ring + (size_t)((*a.step_counter - 1) % a.ring_steps) * a.ring_stride + b : a.rec + slot;
+  if (tid == 0) {
+    const int chosen = a.tok[slot];
+    r->lse = lse;
+    r->logprob = chosen >= 0 && chosen < V ? lg[chosen] - lse : -INFINITY;
+  }
+  if (tid < N) {
+    const unsigned long long key = sk[tid];
+    r->top_ids[tid] = key ? key_id(key) : -1;          // key 0: fewer than top_n entries in the row
+    r->top_logprobs[tid] = key ? key_value(key) - lse : -INFINITY;
+  }
+}
+
+int logprob_blocks(int vocab) {
+  if (vocab <= 0) return 0;
+  const int nblk = (vocab + kSampleChunk - 1) / kSampleChunk;
+  if (nblk * CL_MAX_TOP_LOGPROBS > kSampleChunk) return 0;   // the merge must fit the registers of one CTA
+  return nblk;
+}
+
+int launch_logprobs(const LogprobArgs& a, cudaStream_t st) {
+  static PerDeviceOnce once;
+  const int smem = kSampleChunk * (int)sizeof(unsigned long long);
+  if (once.pending()) {
+    cudaFuncSetAttribute(logprobs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    once.mark();
+  }
+  if (a.batch <= 0 || a.nblk <= 0 || a.nblk != logprob_blocks(a.vocab) || a.top_n < 0 || a.top_n > CL_MAX_TOP_LOGPROBS) return -1;
+  logprobs_kernel<<<dim3(a.nblk, a.batch), kSampleThreads, a.top_n > 0 ? smem : 0, st>>>(a);
+  return cudaGetLastError() == cudaSuccess ? 1 : -1;
+}
+
 int sample_blocks(int vocab) {
   if (vocab <= 0) return 0;
   const int nblk = (vocab + kSampleChunk - 1) / kSampleChunk;

@@ -34,13 +34,17 @@ struct Request {
   // read by the client after `done`
   bool streaming = false;
   std::vector<int32_t> pub;
+  std::vector<LogprobRecord> pub_lp;  // records of `pub` (logprobs requests)
   std::atomic<bool> cancel{false};
   int64_t t_arrive = 0, prefill_ns = 0, decode_ns = 0, t_done = 0;
   uint64_t arrival = 0;
   std::vector<int32_t> full;        // prompt + tokens generated before a preemption: what the (re-)prefill has to process
   size_t prefilled = 0;             // tokens of `full` already in the cache (chunked admission)
   bool dev_sample = false;          // sampled on the device (Engine::sample_qualifies and CL_SCHED_DEVICE_SAMPLE), set at admission
+  int top_n = -1;                   // >= 0: log-probabilities asked for, with top_n alternatives
+  std::vector<LogprobRecord> lp;    // one record per id of `out` (kept across a preemption, like `out`)
   bool greedy() const { return sp.temperature <= 0.f; }
+  bool logprobs() const { return top_n >= 0; }
 };
 
 static void fill_result(const Request& r, cl_result* out, const Tokenizer* tok) {
@@ -60,11 +64,42 @@ static void fill_result(const Request& r, cl_result* out, const Tokenizer* tok) 
   out->n_preempted = r.n_preempted;
 }
 
+static void fill_logprobs(const Request& r, cl_logprobs* out) {
+  memset(out, 0, sizeof *out);
+  const size_t n = r.lp.size(), k = (size_t)std::max(r.top_n, 0);
+  out->n_tokens = (int32_t)n;
+  out->top_n = (int32_t)k;
+  out->logprob = (float*)malloc(sizeof(float) * std::max<size_t>(1, n));
+  if (k) {
+    out->top_ids = (int32_t*)malloc(sizeof(int32_t) * std::max<size_t>(1, n * k));
+    out->top_logprobs = (float*)malloc(sizeof(float) * std::max<size_t>(1, n * k));
+  }
+  for (size_t i = 0; i < n; ++i) {
+    out->logprob[i] = r.lp[i].logprob;
+    for (size_t j = 0; j < k; ++j) {
+      out->top_ids[i * k + j] = r.lp[i].top_ids[j];
+      out->top_logprobs[i * k + j] = r.lp[i].top_logprobs[j];
+    }
+  }
+}
+
 static void publish(Request& r, int32_t id) {
   if (!r.streaming) return;
   std::lock_guard<std::mutex> lk(r.m);
   r.pub.push_back(id);
+  if (r.logprobs()) r.pub_lp.push_back(r.lp.back());
   r.cv.notify_all();
+}
+
+// one generated token: `out`, its record (logprobs requests) and the stream.  `row` (host logits the id was drawn from,
+// may be nullptr): the record's logprob is taken for that id — the kernel saw the step's argmax in d_tok_.
+static void emit_token(Request& r, int32_t id, const LogprobRecord* rec, const float* row) {
+  r.out.push_back(id);
+  if (r.logprobs()) {
+    r.lp.push_back(*rec);
+    if (row) r.lp.back().logprob = row[id] - rec->lse;
+  }
+  publish(r, id);
 }
 
 static bool finished(Request& r, const Tokenizer& tok, int max_seq_len) {
@@ -80,7 +115,8 @@ static int generate_sync(Engine& e, Request& r, const Engine::TokenSink* sink) {
   size_t emitted = 0;
   auto emit = [&]() {
     if (!sink || !sink->fn || r.out.size() <= emitted) return;
-    if (sink->fn(sink->user, r.out.data() + emitted, (int)(r.out.size() - emitted))) r.cancel = true;
+    if (sink->fn(sink->user, r.out.data() + emitted, r.logprobs() ? r.lp.data() + emitted : nullptr, (int)(r.out.size() - emitted)))
+      r.cancel = true;
     emitted = r.out.size();
   };
   std::lock_guard<std::mutex> lk(e.mu_);
@@ -97,6 +133,7 @@ static int generate_sync(Engine& e, Request& r, const Engine::TokenSink* sink) {
   t0 = now_ns();
   std::vector<int32_t> hist(r.prompt);
   int32_t next = 0;
+  LogprobRecord rec;
   if (r.dev_sample) {
     rc = e.sample_setup(r.seq, r.sp, r.prompt.data(), (int)r.prompt.size(), 0);
     if (rc == CL_OK) rc = e.sample_slots(&r.seq, 1, &next);
@@ -104,28 +141,33 @@ static int generate_sync(Engine& e, Request& r, const Engine::TokenSink* sink) {
   } else {
     next = sample_token(logits.data(), V, r.sp, hist.data(), (int)hist.size(), 0);
   }
-  r.out.push_back(next);
+  if (r.logprobs() && (rc = e.logprobs_read(&r.seq, 1, r.top_n, &rec)) != CL_OK) { e.seq_free(r.seq); return rc; }
+  emit_token(r, next, &rec, r.dev_sample ? nullptr : logits.data());
   emit();
+  std::vector<LogprobRecord> recs;
   while (!finished(r, *e.tok, e.cfg.max_seq_len)) {
     if (r.greedy() || r.dev_sample) {
       int room = std::min(r.max_new - (int)r.out.size(), e.cfg.max_seq_len - (int)(r.prompt.size() + r.out.size()));
       int chunk = std::min(room, sink ? 8 : 32);
       std::vector<int32_t> ids(chunk);
+      recs.resize(r.logprobs() ? chunk : 0);
+      LogprobRecord* lp_out = r.logprobs() ? recs.data() : nullptr;
       const uint64_t step = (uint64_t)r.out.size();
-      rc = r.greedy() ? e.decode_greedy(&r.seq, 1, &next, chunk, ids.data(), nullptr)
-                      : e.decode_sample(&r.seq, 1, &next, &r.sp, &step, chunk, ids.data(), nullptr);
+      rc = r.greedy() ? e.decode_greedy(&r.seq, 1, &next, chunk, ids.data(), nullptr, &r.top_n, lp_out)
+                      : e.decode_sample(&r.seq, 1, &next, &r.sp, &step, chunk, ids.data(), nullptr, &r.top_n, lp_out);
       if (rc) break;
       for (int i = 0; i < chunk; ++i) {
-        r.out.push_back(ids[i]);
+        emit_token(r, ids[i], lp_out + i, nullptr);
         if (finished(r, *e.tok, e.cfg.max_seq_len)) break;
       }
       next = r.out.back();
     } else {
       rc = e.decode_step(r.seq, next, logits.data(), nullptr);
+      if (rc == CL_OK && r.logprobs()) rc = e.logprobs_read(&r.seq, 1, r.top_n, &rec);
       if (rc) break;
       hist.push_back(next);
       next = sample_token(logits.data(), V, r.sp, hist.data(), (int)hist.size(), (uint64_t)r.out.size());
-      r.out.push_back(next);
+      emit_token(r, next, &rec, logits.data());
     }
     emit();
   }
@@ -135,8 +177,10 @@ static int generate_sync(Engine& e, Request& r, const Engine::TokenSink* sink) {
   return rc;
 }
 
-int Engine::generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling& sp, cl_result* out, const TokenSink* sink) {
+int Engine::generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling& sp, cl_result* out, const TokenSink* sink,
+                         int top_n, cl_logprobs* lp_out) {
   if (!prompt || n_prompt <= 0 || !out) { set_last_error("empty prompt"); return CL_ERR_INVALID_ARG; }
+  if (top_n > CL_MAX_TOP_LOGPROBS || (top_n >= 0 && !lp_out)) { set_last_error("top_n outside 0..CL_MAX_TOP_LOGPROBS"); return CL_ERR_INVALID_ARG; }
   if (n_prompt >= cfg.max_seq_len) { set_last_error("prompt longer than max_seq_len"); return CL_ERR_TOO_LONG; }
   for (int i = 0; i < n_prompt; ++i)
     if (prompt[i] < 0 || prompt[i] >= cfg.vocab_size) { set_last_error("token id out of range"); return CL_ERR_INVALID_ARG; }
@@ -147,6 +191,7 @@ int Engine::generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling&
   r->max_new = std::min(r->max_new, cfg.max_seq_len - n_prompt);
   r->t_arrive = now_ns();
   r->streaming = sink && sink->fn;
+  r->top_n = top_n < 0 ? -1 : top_n;
   if (!sched_started_) {
     r->status = generate_sync(*this, *r, sink);
     if (r->status == CL_OK) { requests_completed_++; tokens_generated_ += (int64_t)r->out.size(); }
@@ -162,13 +207,15 @@ int Engine::generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling&
     std::unique_lock<std::mutex> lk(r->m);
     size_t seen = 0;
     std::vector<int32_t> fresh;
+    std::vector<LogprobRecord> fresh_lp;
     while (true) {
       r->cv.wait(lk, [&] { return r->done || r->pub.size() > seen; });
       if (r->pub.size() > seen) {
         fresh.assign(r->pub.begin() + seen, r->pub.end());
+        if (r->logprobs()) fresh_lp.assign(r->pub_lp.begin() + seen, r->pub_lp.end());
         seen = r->pub.size();
         lk.unlock();                       // the callback runs on this (the caller's) thread, outside every lock
-        if (sink->fn(sink->user, fresh.data(), (int)fresh.size())) r->cancel = true;
+        if (sink->fn(sink->user, fresh.data(), r->logprobs() ? fresh_lp.data() : nullptr, (int)fresh.size())) r->cancel = true;
         lk.lock();
         continue;
       }
@@ -181,6 +228,7 @@ int Engine::generate_ids(const int32_t* prompt, int n_prompt, const cl_sampling&
     return r->status;
   }
   fill_result(*r, out, tok.get());
+  if (r->logprobs()) fill_logprobs(*r, lp_out);
   return CL_OK;
 }
 
@@ -217,6 +265,7 @@ void Engine::scheduler_main() {
   std::vector<int32_t> toks(max_seqs_);
   std::vector<int> slots;
   std::vector<int> last_slots;
+  std::vector<cl_seq_t> lp_slots;
   {
     std::lock_guard<std::mutex> elk(mu_);
     {
@@ -311,6 +360,13 @@ void Engine::scheduler_main() {
           if (rc == CL_OK) rc = sample_slots(dev.data(), (int)dev.size(), nullptr);
         }
         if (rc == CL_OK) {
+          // the first tokens' log-probabilities: one launch over the group's rows that asked
+          std::vector<cl_seq_t> lps;
+          int lp_n = -1;
+          for (auto& r : group) if (r->logprobs()) { lps.push_back(r->seq); lp_n = std::max(lp_n, r->top_n); }
+          if (!lps.empty()) rc = logprobs_enqueue(lps.data(), (int)lps.size(), lp_n);
+        }
+        if (rc == CL_OK) {
           cudaMemcpyAsync(toks.data(), d_tok_, (size_t)max_seqs_ * 4, cudaMemcpyDeviceToHost, stream_);
           if (cudaStreamSynchronize(stream_) != cudaSuccess) rc = CL_ERR_CUDA;
         }
@@ -323,14 +379,14 @@ void Engine::scheduler_main() {
             r->prefill_ns += pdt;
             r->prefilled = r->full.size();
             int32_t next = toks[r->seq];                       // greedy: the device argmax of the pass; device-sampled: the draw
-            if (!r->greedy() && !r->dev_sample) {
+            const bool host = !r->greedy() && !r->dev_sample;
+            if (host) {
               read_logits(r->seq, logits.data());
               next = sample_token(logits.data(), V, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
               cudaMemcpyAsync(d_tok_ + r->seq, &next, 4, cudaMemcpyHostToDevice, stream_);
               cudaStreamSynchronize(stream_);
             }
-            r->out.push_back(next);
-            publish(*r, next);
+            emit_token(*r, next, r->logprobs() ? &lp_host(r->seq) : nullptr, host ? logits.data() : nullptr);
             if (finished(*r, *tok, cfg.max_seq_len)) {
               seq_free(r->seq);
               requests_completed_++;
@@ -404,8 +460,11 @@ void Engine::scheduler_main() {
       } else {
         next = sample_token(logits.data(), V, r->sp, r->full.data(), (int)r->full.size(), (uint64_t)r->out.size());
       }
-      r->out.push_back(next);
-      publish(*r, next);
+      LogprobRecord rec;
+      if (r->logprobs() && (rc = logprobs_read(&r->seq, 1, r->top_n, &rec)) != CL_OK) {
+        seq_free(r->seq); r->seq = -1; complete(r, rc, get_last_error()); continue;
+      }
+      emit_token(*r, next, &rec, r->dev_sample ? nullptr : logits.data());
       if (!r->greedy() && !r->dev_sample) cudaMemcpyAsync(d_tok_ + r->seq, &r->out.back(), 4, cudaMemcpyHostToDevice, stream_);
       if (finished(*r, *tok, cfg.max_seq_len)) {
         seq_free(r->seq);
@@ -472,6 +531,11 @@ void Engine::scheduler_main() {
     // the device sampler overwrites the step's argmax of the device-sampled slots (one launch for the whole batch)
     if (rc == CL_OK && std::any_of(active_.begin(), active_.end(), [](const std::shared_ptr<Request>& r) { return r->dev_sample; }))
       rc = launch_sampler(B, d_slots_, false);
+    // log-probabilities of the rows that asked (one launch; nothing at all when no row did)
+    lp_slots.clear();
+    int lp_n = -1;
+    for (auto& r : active_) if (r->logprobs()) { lp_slots.push_back(r->seq); lp_n = std::max(lp_n, r->top_n); }
+    if (rc == CL_OK && !lp_slots.empty()) rc = logprobs_enqueue(lp_slots.data(), (int)lp_slots.size(), lp_n);
     if (rc == CL_OK) {
       cudaMemcpyAsync(toks.data(), d_tok_, (size_t)max_seqs_ * 4, cudaMemcpyDeviceToHost, stream_);
       // Batched steps last 3.5-6 ms: wait on a blocking-sync event instead of spinning in cudaStreamSynchronize, so that
@@ -494,14 +558,14 @@ void Engine::scheduler_main() {
       st.history.push_back(r->out.back());
       st.len += 1;
       int32_t next = toks[r->seq];
-      if (!r->greedy() && !r->dev_sample) {
+      const bool host = !r->greedy() && !r->dev_sample;
+      if (host) {
         read_logits(r->seq, logits.data());
         next = sample_token(logits.data(), V, r->sp, st.history.data(), (int)st.history.size(), (uint64_t)r->out.size());
         cudaMemcpyAsync(d_tok_ + r->seq, &next, 4, cudaMemcpyHostToDevice, stream_);
         cudaStreamSynchronize(stream_);
       }
-      r->out.push_back(next);
-      publish(*r, next);
+      emit_token(*r, next, r->logprobs() ? &lp_host(r->seq) : nullptr, host ? logits.data() : nullptr);
     }
     const int64_t dt = now_ns() - t0;
     for (auto& r : active_) r->decode_ns += dt;

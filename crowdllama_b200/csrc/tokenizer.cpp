@@ -173,6 +173,10 @@ class HfBpeTokenizer : public Tokenizer {
   bool load(const std::string& path, const std::string& chat_family, std::string* err);
   std::vector<int32_t> encode(const std::string& text, bool add_bos) const override;
   std::string decode_bytes(const std::vector<int32_t>& ids) const override;
+  std::string token_bytes(int id) const override {
+    if (id >= 0 && id < (int)id_to_tok_.size() && special_[id]) return id_to_tok_[id];   // added-token content
+    return decode_bytes({id});
+  }
   int bos() const override { return bos_; }
   int eos() const override { return eos_; }
   bool is_stop(int id) const override { return id == eos_ || id == eot_; }

@@ -21,6 +21,8 @@ CL_ERR_INVALID_ARG, CL_ERR_NO_DEVICE, CL_ERR_CUDA, CL_ERR_OOM, CL_ERR_UNKNOWN_MO
 # device sampler limits (include/clengine.h CL_SAMPLE_MAX_TOP_K / CL_SAMPLE_MAX_WINDOW)
 SAMPLE_MAX_TOP_K = 128
 SAMPLE_MAX_WINDOW = 64
+# most alternatives a log-probability entry carries (include/clengine.h CL_MAX_TOP_LOGPROBS)
+MAX_TOP_LOGPROBS = 20
 
 KINDS = dict(EMBED=0, LM_HEAD=1, FINAL_NORM=2, ATTN_NORM=3, WQ=4, WK=5, WV=6, WO=7, FFN_NORM=8, WGATE=9, WUP=10,
              WDOWN=11)
@@ -57,6 +59,11 @@ class Result(C.Structure):
                 ("n_preempted", C.c_int32)]
 
 
+class Logprobs(C.Structure):
+    _fields_ = [("n_tokens", C.c_int32), ("top_n", C.c_int32), ("logprob", C.POINTER(C.c_float)),
+                ("top_ids", C.POINTER(C.c_int32)), ("top_logprobs", C.POINTER(C.c_float))]
+
+
 class Stats(C.Structure):
     _fields_ = [("tokens_per_sec", C.c_double), ("load", C.c_double), ("queue_depth", C.c_int32),
                 ("active_seqs", C.c_int32), ("kv_pages_total", C.c_int32), ("kv_pages_used", C.c_int32),
@@ -70,12 +77,13 @@ class Stats(C.Structure):
 EXPORTS = [
     "cl_abi_version", "cl_strerror", "cl_last_error", "cl_default_engine_config", "cl_default_sampling",
     "cl_greedy_sampling", "cl_sample_token", "cl_model_preset", "cl_engine_create", "cl_engine_destroy", "cl_engine_model_config",
-    "cl_engine_stats", "cl_engine_set_tensor", "cl_checkpoint_info", "cl_generate", "cl_generate_ids", "cl_generate_stream", "cl_result_free",
+    "cl_engine_stats", "cl_engine_set_tensor", "cl_checkpoint_info", "cl_generate", "cl_generate_ids", "cl_generate_ids_logprobs",
+    "cl_logprobs_free", "cl_generate_stream", "cl_result_free",
     "cl_handle_message", "cl_handle_message_stream", "cl_buffer_free", "cl_tokenize", "cl_detokenize", "cl_seq_create", "cl_seq_free",
     "cl_seq_len", "cl_prefill", "cl_prefill_batch", "cl_decode_step", "cl_decode_greedy", "cl_decode_greedy_batch", "cl_decode_sample_batch", "cl_decode_step_batch", "cl_seq_fake_fill",
     "cl_time_dominant_kernel", "cl_debug_kv", "cl_debug_hidden", "cl_debug_timeline",
     "cl_op_gemv", "cl_op_gemv_residual", "cl_op_rmsnorm_gemv", "cl_op_rmsnorm_gateup", "cl_op_qkv_rope_append", "cl_op_attn_decode",
-    "cl_op_gemm_bf16", "cl_op_attn_prefill", "cl_op_attn_prefill_variant", "cl_op_sample", "cl_op_synth_weights", "cl_kvpool_create", "cl_kvpool_destroy",
+    "cl_op_gemm_bf16", "cl_op_attn_prefill", "cl_op_attn_prefill_variant", "cl_op_sample", "cl_op_logprobs", "cl_op_synth_weights", "cl_kvpool_create", "cl_kvpool_destroy",
     "cl_kvpool_reserve", "cl_kvpool_release", "cl_kvpool_pages_of", "cl_kvpool_free_pages", "cl_kvpool_used_pages",
     "cl_tokenizer_load", "cl_tokenizer_free", "cl_tokenizer_encode", "cl_tokenizer_decode", "cl_tokenizer_info", "cl_engine_load_tokenizer",
 ]
@@ -114,6 +122,8 @@ def lib():
         "cl_checkpoint_info": (C.c_int, [C.c_char_p, P(ModelConfig), P(i32), P(i64)]),
         "cl_generate": (C.c_int, [vp, C.c_char_p, C.c_char_p, sz, P(Sampling), P(Result)]),
         "cl_generate_ids": (C.c_int, [vp, vp, i32, P(Sampling), P(Result)]),
+        "cl_generate_ids_logprobs": (C.c_int, [vp, vp, i32, P(Sampling), i32, P(Result), P(Logprobs)]),
+        "cl_logprobs_free": (None, [P(Logprobs)]),
         "cl_generate_stream": (C.c_int, [vp, C.c_char_p, C.c_char_p, sz, P(Sampling), TOKEN_CB, vp, P(Result)]),
         "cl_handle_message_stream": (C.c_int, [vp, C.c_char_p, sz, P(Sampling), FRAME_CB, vp]),
         "cl_result_free": (None, [P(Result)]),
@@ -147,6 +157,7 @@ def lib():
         "cl_op_attn_prefill": (C.c_int, [C.c_int, vp, vp, vp, i32, i32, i32, i32, vp]),
         "cl_op_attn_prefill_variant": (C.c_int, [C.c_int, C.c_int, vp, vp, vp, i32, i32, i32, i32, vp, i32, P(f32)]),
         "cl_op_sample": (C.c_int, [C.c_int, vp, i32, i32, P(Sampling), vp, vp, vp, vp, i32, P(f32)]),
+        "cl_op_logprobs": (C.c_int, [C.c_int, vp, i32, i32, vp, i32, vp, vp, vp, i32, P(f32)]),
         "cl_op_synth_weights": (C.c_int, [C.c_int, u64, i32, i64, f32, vp]),
         "cl_tokenizer_load": (C.c_int, [C.c_char_p, C.c_char_p, P(vp)]),
         "cl_tokenizer_free": (None, [vp]),
@@ -239,6 +250,10 @@ def ollama_default_sampling(seed: int = 0, max_new_tokens: int = -1) -> Sampling
 
 
 class GenerateResult:
+    """With log-probabilities (generate_ids(..., top_logprobs=N)): logprob [n_generated] float32, top_ids / top_logprobs
+    [n_generated][N]; otherwise those three are None."""
+    logprob = top_ids = top_logprobs = None
+
     def __init__(self, r: Result):
         self.text = C.string_at(r.text, r.text_len).decode("utf-8", errors="replace") if r.text else ""
         self.done_reason = C.string_at(r.done_reason).decode() if r.done_reason else ""
@@ -412,14 +427,33 @@ class Engine:
         return out.reshape(-1, 4)
 
     # ---- request level ---------------------------------------------------------------------------
-    def generate_ids(self, prompt_ids, sampling: Sampling) -> GenerateResult:
+    def generate_ids(self, prompt_ids, sampling: Sampling, top_logprobs: int | None = None) -> GenerateResult:
+        """top_logprobs (0..MAX_TOP_LOGPROBS): also return the log-probability of every generated token with that many
+        alternatives (cl_generate_ids_logprobs); None: cl_generate_ids."""
         ids = np.ascontiguousarray(prompt_ids, dtype=np.int32)
         r = Result()
-        _check(lib().cl_generate_ids(self._h, _ptr(ids), len(ids), C.byref(sampling), C.byref(r)), "cl_generate_ids")
+        if top_logprobs is None:
+            _check(lib().cl_generate_ids(self._h, _ptr(ids), len(ids), C.byref(sampling), C.byref(r)), "cl_generate_ids")
+            try:
+                return GenerateResult(r)
+            finally:
+                lib().cl_result_free(C.byref(r))
+        lp = Logprobs()
+        _check(lib().cl_generate_ids_logprobs(self._h, _ptr(ids), len(ids), C.byref(sampling), int(top_logprobs), C.byref(r), C.byref(lp)),
+               "cl_generate_ids_logprobs")
         try:
-            return GenerateResult(r)
+            g = GenerateResult(r)
+            n, k = lp.n_tokens, lp.top_n
+            g.logprob = np.ctypeslib.as_array(lp.logprob, shape=(n,)).copy() if n else np.zeros(0, np.float32)
+            if k and n:
+                g.top_ids = np.ctypeslib.as_array(lp.top_ids, shape=(n * k,)).reshape(n, k).copy()
+                g.top_logprobs = np.ctypeslib.as_array(lp.top_logprobs, shape=(n * k,)).reshape(n, k).copy()
+            else:
+                g.top_ids, g.top_logprobs = np.zeros((n, k), np.int32), np.zeros((n, k), np.float32)
+            return g
         finally:
             lib().cl_result_free(C.byref(r))
+            lib().cl_logprobs_free(C.byref(lp))
 
     def generate(self, model: str, prompt: str, sampling: Sampling | None = None) -> GenerateResult:
         r = Result()
@@ -624,6 +658,23 @@ def op_sample(logits, samplings, windows, steps, iters=0, device=0):
     _check(lib().cl_op_sample(device, _ptr(lg), n, v, sps, _ptr(win), _ptr(nwin), _ptr(st), _ptr(ids), iters, C.byref(ms)),
            "cl_op_sample")
     return ids, ms.value
+
+
+def op_logprobs(logits, chosen, top_n, iters=0, device=0):
+    """cl_op_logprobs: logprobs_kernel on host logits [n_rows][vocab] with chosen[n_rows] the emitted ids.  Returns
+    (logprob [n_rows], top_ids [n_rows][top_n], top_logprobs [n_rows][top_n], mean ms of `iters` timed launches or 0)."""
+    lg = np.ascontiguousarray(logits, dtype=np.float32)
+    n, v = lg.shape
+    ch = np.ascontiguousarray(chosen, dtype=np.int32)
+    if ch.shape != (n,):
+        raise ValueError("chosen needs one id per row")
+    lp = np.empty(n, np.float32)
+    ids = np.empty((n, max(top_n, 0)), np.int32)
+    tl = np.empty((n, max(top_n, 0)), np.float32)
+    ms = C.c_float(0)
+    _check(lib().cl_op_logprobs(device, _ptr(lg), n, v, _ptr(ch), int(top_n), _ptr(lp), _ptr(ids) if top_n > 0 else None,
+                                _ptr(tl) if top_n > 0 else None, iters, C.byref(ms)), "cl_op_logprobs")
+    return lp, ids, tl, ms.value
 
 
 def op_synth_weights(seed, key, n, scale, device=0):

@@ -3,7 +3,8 @@
 Mirrors pkg/gateway/gateway.go: POST /api/chat (handleChat :168-231 → FindBestWorker :191 → RequestInference
 :243-293) and GET /api/health (:453-461).  SURVEY.md §8f rows 3-4 on top: POST /api/generate (BASELINE.json names
 it, the reference gateway lacks it, gateway.go:87-88), the Ollama `options` object passed through to the worker
-(GenerateRequest.options), and `"stream": true` answered as NDJSON lines (one per worker frame).  Worker discovery (DHT provider lookup + metadata fetch,
+(GenerateRequest.options), and `"stream": true` answered as NDJSON lines (one per worker frame); Ollama's top-level
+`logprobs` / `top_logprobs` travel as options 9 / 10 and come back per token in GenerateResponse.logprobs (`logprobs_json`).  Worker discovery (DHT provider lookup + metadata fetch,
 internal/discovery/discovery.go:278-366) is replaced by a static address list whose metadata is polled
 over the metadata protocol — the routing rule itself (peermanager FindBestWorker) is `router.find_best_worker`.
 Quirks kept: only messages[0].content is forwarded (gateway.go:209); handler errors arrive as assistant
@@ -23,6 +24,16 @@ from . import handler as H
 from .pbwire import read_length_prefixed_pb, write_length_prefixed_pb
 from .router import Resource, find_best_worker
 from .worker import INFERENCE_PROTOCOL, METADATA_PROTOCOL, _Stream
+
+MAX_TOP_LOGPROBS = 20     # include/clengine.h CL_MAX_TOP_LOGPROBS
+
+
+def logprobs_json(entries) -> list:
+    """GenerateResponse.logprobs (pb.TokenLogprob) -> the reply's "logprobs" array, the shape of Ollama's API
+    documentation: one object per generated token with its text, log-probability, UTF-8 bytes and alternatives."""
+    def one(t):
+        return {"token": t.token.decode("utf-8", "replace"), "logprob": t.logprob, "bytes": list(t.token)}
+    return [{**one(t), "top_logprobs": [one(a) for a in t.top_logprobs]} for t in entries]
 
 
 class PeerTable:
@@ -141,6 +152,13 @@ class _Handler(BaseHTTPRequestHandler):
         if not chat and req.get("raw"):
             options = options or GenerateOptions()
             options.raw = True
+        want_logprobs = bool(req.get("logprobs", False))
+        top_logprobs = req.get("top_logprobs", 0)
+        if isinstance(top_logprobs, bool) or not isinstance(top_logprobs, int) or not 0 <= top_logprobs <= MAX_TOP_LOGPROBS:
+            return self._json(400, {"error": f"top_logprobs must be an integer within 0..{MAX_TOP_LOGPROBS}"})
+        if want_logprobs:
+            options = options or GenerateOptions()
+            options.logprobs, options.top_logprobs = True, top_logprobs
         stream = bool(req.get("stream", False))
         addr, worker = self.server.table.best(model)
         if worker is None:                                                # gateway.go:192-199
@@ -155,6 +173,8 @@ class _Handler(BaseHTTPRequestHandler):
                      "done": g.done}
             else:
                 o = {"model": g.model or model, "created_at": now, "response": g.response, "done": g.done}
+            if want_logprobs:
+                o["logprobs"] = logprobs_json(g.logprobs)
             if g.done:
                 o["done_reason"] = g.done_reason
             return o

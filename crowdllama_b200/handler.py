@@ -71,8 +71,10 @@ def worker_api_handler(engine: "eng.Engine", sampling: "eng.Sampling | None" = N
         return generate_req
 
     def _raw(generate_req) -> bool:
-        # raw = "do not apply the chat template": only the byte-level entry points of libclengine know how
-        return bool(generate_req.options and generate_req.options.raw and hasattr(engine, "handle_message_stream"))
+        # raw = "do not apply the chat template", logprobs = GenerateResponse.logprobs: only the byte-level entry points
+        # of libclengine know how
+        o = generate_req.options
+        return bool(o and (o.raw or o.logprobs) and hasattr(engine, "handle_message_stream"))
 
     def handler(ctx, req: BaseMessage) -> BaseMessage:
         generate_req = _request(req)

@@ -14,10 +14,14 @@ FIELDS = {
     "GenerateRequest": {"model": 1, "prompt": 2, "stream": 3, "options": 4},
     # EXTENSION (SURVEY.md §8f row 3): request options the reference's wire cannot express (api.go:193-197);
     # every field has explicit presence (proto3 `optional`): temperature 0 = greedy is not "unset"
+    # logprobs / top_logprobs: the log-probabilities of the generated tokens (Ollama's top-level request fields)
     "GenerateOptions": {"seed": 1, "temperature": 2, "top_k": 3, "top_p": 4, "repeat_penalty": 5, "repeat_last_n": 6,
-                        "num_predict": 7, "raw": 8},
+                        "num_predict": 7, "raw": 8, "logprobs": 9, "top_logprobs": 10},
+    # EXTENSION: logprobs = one TokenLogprob per token id the frame covers (a peer without it skips field 8)
     "GenerateResponse": {"model": 1, "created_at": 2, "response": 3, "done": 4, "done_reason": 5, "worker_id": 6,
-                         "total_duration": 7},
+                         "total_duration": 7, "logprobs": 8},
+    "TokenLogprob": {"token": 1, "logprob": 2, "top_logprobs": 3},
+    "TopLogprob": {"token": 1, "logprob": 2},
     "Timestamp": {"seconds": 1, "nanos": 2},
 }
 
@@ -77,6 +81,7 @@ def _fields(b: bytes):
 import struct
 
 _OPT_FLOAT = ("temperature", "top_p", "repeat_penalty")
+_OPT_BOOL = ("raw", "logprobs")
 
 
 @dataclass
@@ -90,6 +95,8 @@ class GenerateOptions:
     repeat_last_n: int | None = None
     num_predict: int | None = None
     raw: bool | None = None
+    logprobs: bool | None = None
+    top_logprobs: int | None = None
 
     def encode(self) -> bytes:
         F, out = FIELDS["GenerateOptions"], b""
@@ -114,8 +121,8 @@ class GenerateOptions:
             if name in _OPT_FLOAT and wt == 5:
                 setattr(m, name, struct.unpack("<f", v)[0])
             elif name not in _OPT_FLOAT and wt == 0:
-                if name == "raw":
-                    m.raw = bool(v)
+                if name in _OPT_BOOL:
+                    setattr(m, name, bool(v))
                 elif name == "seed":
                     m.seed = v
                 else:
@@ -138,6 +145,56 @@ class GenerateOptions:
 
     def is_empty(self) -> bool:
         return all(getattr(self, k) is None for k in FIELDS["GenerateOptions"])
+
+
+def _f32(fno: int, v: float) -> bytes:
+    return _varint(fno << 3 | 5) + struct.pack("<f", float(v)) if v != 0.0 else b""
+
+
+@dataclass
+class TopLogprob:
+    token: bytes = b""              # the surface bytes of the id on its own
+    logprob: float = 0.0
+
+    def encode(self) -> bytes:
+        F = FIELDS["TopLogprob"]
+        return (_ld(F["token"], self.token) if self.token else b"") + _f32(F["logprob"], self.logprob)
+
+    @classmethod
+    def decode(cls, b: bytes) -> "TopLogprob":
+        F, m = FIELDS["TopLogprob"], cls()
+        for f, wt, v in _fields(b):
+            if f == F["token"] and wt == 2:
+                m.token = bytes(v)
+            elif f == F["logprob"] and wt == 5:
+                m.logprob = struct.unpack("<f", v)[0]
+        return m
+
+
+@dataclass
+class TokenLogprob:
+    token: bytes = b""
+    logprob: float = 0.0
+    top_logprobs: list = field(default_factory=list)    # [TopLogprob]
+
+    def encode(self) -> bytes:
+        F = FIELDS["TokenLogprob"]
+        out = (_ld(F["token"], self.token) if self.token else b"") + _f32(F["logprob"], self.logprob)
+        for t in self.top_logprobs:
+            out += _ld(F["top_logprobs"], t.encode())
+        return out
+
+    @classmethod
+    def decode(cls, b: bytes) -> "TokenLogprob":
+        F, m = FIELDS["TokenLogprob"], cls()
+        for f, wt, v in _fields(b):
+            if f == F["token"] and wt == 2:
+                m.token = bytes(v)
+            elif f == F["logprob"] and wt == 5:
+                m.logprob = struct.unpack("<f", v)[0]
+            elif f == F["top_logprobs"] and wt == 2:
+                m.top_logprobs.append(TopLogprob.decode(v))
+        return m
 
 
 @dataclass
@@ -185,6 +242,7 @@ class GenerateResponse:
     done_reason: str = ""
     worker_id: str = ""
     total_duration: int = 0
+    logprobs: list = field(default_factory=list)        # [TokenLogprob], one per token id of this frame
 
     def encode(self) -> bytes:
         F, T = FIELDS["GenerateResponse"], FIELDS["Timestamp"]
@@ -208,6 +266,8 @@ class GenerateResponse:
             out += _ld(F["worker_id"], self.worker_id.encode())
         if self.total_duration:
             out += _varint(F["total_duration"] << 3) + _varint(self.total_duration)
+        for t in self.logprobs:
+            out += _ld(F["logprobs"], t.encode())
         return out
 
     @classmethod
@@ -232,6 +292,8 @@ class GenerateResponse:
                 m.worker_id = v.decode("utf-8", "replace")
             elif f == F["total_duration"] and wt == 0:
                 m.total_duration = v if v < 1 << 63 else v - (1 << 64)
+            elif f == F["logprobs"] and wt == 2:
+                m.logprobs.append(TokenLogprob.decode(v))
         return m
 
 

@@ -116,6 +116,23 @@ typedef struct cl_sampling {
 #define CL_SAMPLE_MAX_TOP_K 128
 #define CL_SAMPLE_MAX_WINDOW 64
 
+/* Log-probabilities of the generated tokens (Ollama `logprobs` / `top_logprobs`).  The numbers describe the model's raw
+ * next-token distribution, log_softmax of the fp32 logits of the step, before the repeat penalty, the temperature and
+ * the top-k / top-p cuts; they are the same for greedy and sampled requests.  For generated token i:
+ *   logprob[i]                          = logits[token_ids[i]] - logsumexp(logits)
+ *   top_ids[i * top_n + j], top_logprobs[i * top_n + j], j < top_n
+ *                                       = the top_n most likely ids, value descending, then id ascending
+ * Computed on the device (logprobs_kernel), one launch per step over the rows that asked; bit-reproducible. */
+#define CL_MAX_TOP_LOGPROBS 20
+typedef struct cl_logprobs {
+  int32_t n_tokens;        /* == cl_result.n_generated */
+  int32_t top_n;
+  float* logprob;          /* [n_tokens], malloc'd */
+  int32_t* top_ids;        /* [n_tokens][top_n], malloc'd (NULL when top_n == 0) */
+  float* top_logprobs;     /* [n_tokens][top_n], malloc'd (NULL when top_n == 0) */
+} cl_logprobs;
+void cl_logprobs_free(cl_logprobs* l);
+
 typedef struct cl_result {
   char* text;            /* NUL-terminated UTF-8, malloc'd */
   size_t text_len;
@@ -197,6 +214,11 @@ int cl_generate(cl_engine* e, const char* model, const char* prompt, size_t prom
 int cl_generate_ids(cl_engine* e, const int32_t* prompt_ids, int32_t n_prompt,
                     const cl_sampling* s, cl_result* out);
 void cl_result_free(cl_result* r);
+/* cl_generate_ids with the log-probabilities of every generated token (CL_MAX_TOP_LOGPROBS above): lp receives one
+ * entry per id of out->token_ids, each with its top_n (0..CL_MAX_TOP_LOGPROBS, else CL_ERR_INVALID_ARG) most likely
+ * alternatives; free it with cl_logprobs_free.  The ids are the ones cl_generate_ids returns for the same request. */
+int cl_generate_ids_logprobs(cl_engine* e, const int32_t* prompt_ids, int32_t n_prompt, const cl_sampling* s,
+                             int32_t top_n, cl_result* out, cl_logprobs* lp);
 
 /* Streaming variant of cl_generate (SURVEY.md §8f row 4; the reference rejects stream:true, api.go:155).
  * cb runs on the CALLING thread (cgo-safe) with each batch of new tokens: text = UTF-8 delta that later tokens
@@ -210,7 +232,9 @@ int cl_generate_stream(cl_engine* e, const char* model, const char* prompt, size
  * Done=true frame with done_reason — each handed to cb (the host writes them length-prefixed to the stream,
  * pbwire.go:14-33).  Without stream: exactly one Done=true frame.  GenerateRequest.options (field 4, the proto
  * extension of §8f row 3: seed, temperature, top_k, top_p, repeat_penalty, repeat_last_n, num_predict, raw)
- * override `s` field by field in both entry points. */
+ * override `s` field by field in both entry points.  With options.logprobs (field 9) every GenerateResponse carries
+ * GenerateResponse.logprobs (field 8): one TokenLogprob per token id the frame covers, with options.top_logprobs
+ * (field 10, 0..CL_MAX_TOP_LOGPROBS, else CL_ERR_INVALID_ARG) alternatives each. */
 typedef int (*cl_frame_cb)(void* user, const uint8_t* msg, size_t len);
 int cl_handle_message_stream(cl_engine* e, const uint8_t* req, size_t req_len, const cl_sampling* s,
                              cl_frame_cb cb, void* user);
@@ -330,6 +354,12 @@ int cl_op_attn_prefill_variant(int device, int variant, const uint16_t* q, const
 int cl_op_sample(int device, const float* logits, int32_t n_rows, int32_t vocab, const cl_sampling* s,
                  const int32_t* windows, const int32_t* n_window, const uint64_t* steps, int32_t* ids_out, int32_t iters,
                  float* ms);
+/* logprobs_kernel on host logits [n_rows][vocab] fp32 with chosen[n_rows] the emitted ids: logprob[r] =
+ * logits[r][chosen[r]] - logsumexp(logits[r]); top_ids / top_logprobs [n_rows][top_n] (may be NULL when top_n == 0) the
+ * top_n best entries of each row, value descending, then id ascending.  top_n outside 0..CL_MAX_TOP_LOGPROBS:
+ * CL_ERR_INVALID_ARG.  iters > 0: also time that many launches over copies of the logits larger than L2 (*ms: mean). */
+int cl_op_logprobs(int device, const float* logits, int32_t n_rows, int32_t vocab, const int32_t* chosen, int32_t top_n,
+                   float* logprob, int32_t* top_ids, float* top_logprobs, int32_t iters, float* ms);
 /* synthetic weight generator (device kernel) -> host copy, for known-answer tests */
 int cl_op_synth_weights(int device, uint64_t seed, int32_t tensor_key, int64_t n, float scale,
                         uint16_t* out_bf16);
